@@ -3,6 +3,8 @@
 
     python bench.py --gpus N --steps K --warmup W            (our arm, one process per GPU)
     python bench.py --impl reference --gpus N --steps K ...   (reference CPU arm, rank 0 only)
+    python bench.py ... --dump-outputs DIR                    (also write the last timed step's outputs as DIR/*.npy;
+                                                               the inputs are seeded, so two builds compare file by file)
 
 Workload (every N, strong scaling): BASELINE.json config 5 — ONE 16384x16384 synthetic mosaic cut into 361 tiles
 of 1024 px with 128 px overlap, partitioned over the N ranks in contiguous blocks. A "step" is one pass over the
@@ -64,7 +66,14 @@ def parse():
     ap.add_argument("--features-layout", default="channels_last", choices=["channels_last", "nchw"],
                     help="memory format of the synthetic FPN maps: channels_last = what the channels_last backbone that "
                          "patch_model sets up produces (gathered in place); nchw = torchvision's default layout")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def peaks():
@@ -76,12 +85,13 @@ def peaks():
 
 
 _SAMPLER_SRC = r"""
-import sys, time
+import os, sys, time
 import pynvml as nv
+parent = int(sys.argv[2])           # the benchmark's pid, passed in: it may be gone before this line runs
 nv.nvmlInit()
 h = nv.nvmlDeviceGetHandleByIndex(int(sys.argv[1]))
 print("max", nv.nvmlDeviceGetMaxClockInfo(h, nv.NVML_CLOCK_SM), flush=True)
-while True:
+while os.getppid() == parent:       # ends with the benchmark, also when that one stops on an error
     print(time.time(), nv.nvmlDeviceGetClockInfo(h, nv.NVML_CLOCK_SM), nv.nvmlDeviceGetCurrentClocksEventReasons(h), flush=True)
     time.sleep(0.001)
 """
@@ -96,7 +106,7 @@ class ClockSampler:
         import tempfile
         self.out = tempfile.TemporaryFile(mode="w+")
         try:
-            self.proc = subprocess.Popen([sys.executable, "-c", _SAMPLER_SRC, str(index)], stdout=self.out,
+            self.proc = subprocess.Popen([sys.executable, "-c", _SAMPLER_SRC, str(index), str(os.getpid())], stdout=self.out,
                                          stderr=subprocess.DEVNULL)
         except Exception:
             self.proc = None
@@ -173,6 +183,39 @@ def roi_align_algorithmic_bytes(proposals, counts, grids, thresholds, scales, ch
         touched += int(m.sum())
     k_live = int(live.sum())
     return 20 * k_live + 4 * channels * pooled * pooled * k_live + 4 * channels * touched, k_live, touched
+
+
+def dump_outputs(out_dir, gathered, state, res, rank=0, world=1, budget=60_000_000, seed=0):
+    """Writes what one mosaic pass hands its caller as out_dir/<name>.npy, in float32 where that holds the values
+    exactly and float64 otherwise: the gathered detection rows [rows, 6] (box, score, label or -1), the seam NMS
+    state of every row (1 kept, 2 suppressed, 3 ignored) and the rank's crops (annotation bounds, integer
+    rectangles, source rows, byte offsets). The crop bytes (~2 GB per pass at the default size) do not fit the
+    budget: a fixed, seeded sample of byte positions goes to crop_pixel_index and the bytes there to crop_pixels.
+    With several ranks the gathered rows and the seam state are the same on every rank and rank 0 alone writes
+    them; every rank writes its own crop arrays as <name>.rank<r>.npy within an equal share of what is left.
+    `budget` counts the arrays of all ranks together and keeps all files, headers included, under 64 MB.
+    Returns {file name without .npy: array} of what this rank wrote."""
+    import numpy as np
+    import torch
+    shared = {"gathered_rows": gathered.float(), "seam_state": state.float()}
+    own = {"crop_xywh": res["xywh"].float(), "crop_rects": res["rects"].float(), "crop_src_rows": res["src"].float(),
+           "crop_offsets": res["offsets"].double()}
+    shared, own = ({k: v.cpu().numpy() for k, v in d.items()} for d in (shared, own))
+    left = (budget - sum(a.nbytes for a in shared.values())) // world - sum(a.nbytes for a in own.values())
+    if left < 0:
+        raise SystemExit(f"--dump-outputs: the detection arrays alone exceed {budget} bytes")
+    pixels = res["pixels"]
+    k = min(pixels.numel(), left // 12)                          # 8 B index + 4 B value per sampled byte
+    idx = np.sort(np.random.default_rng(seed).choice(pixels.numel(), k, replace=False)) if k < pixels.numel() else np.arange(k)
+    own["crop_pixel_index"] = idx.astype(np.float64)
+    own["crop_pixels"] = pixels[torch.from_numpy(idx).to(pixels.device)].float().cpu().numpy()
+    suffix = f".rank{rank}" if world > 1 else ""
+    out = dict(shared) if rank == 0 else {}
+    out.update({name + suffix: a for name, a in own.items()})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return out
 
 
 # ----------------------------------------------------------------------------------------------
@@ -523,6 +566,8 @@ def run_ours(args):
     recording[0] = False
     clocks = sampler.summary(wall0, time.time()) if rank == 0 else None
     tma_used = _lib.load().mb_roi_align_tma_launches() - tma0
+    if args.dump_outputs:                                    # before the legs below overwrite the plan's buffers
+        dump_outputs(args.dump_outputs, plan.gathered, plan.seam.state, plan.results(), rank, world)
     t = torch.tensor([float(my_dets), float(my_crop_bytes)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.SUM)
