@@ -293,6 +293,21 @@ int mb_roi_align_backward(const float* grad, const float* rois, int64_t num_rois
  * ------------------------------------------------------------------------------------ */
 int mb_paste_masks(const float* masks, const float* boxes, int64_t num_masks, int32_t mask_side,
                    int32_t padding, int32_t im_h, int32_t im_w, float* out, mb_stream_t stream);
+/* Per-crop instance masks: paste_masks_in_image (tv:models/detection/roi_heads.py:375-501) evaluated only
+ * at the pixels of the crop rectangles of mb_crop_plan, thresholded. Crop j of slot s = src[j] with
+ * rect (x, y, w, h): mask_j[r, c] = 255 if paste(mask_probs[s], paste_boxes[s], frame (fh, fw))
+ * [y + r - y0, x + c - x0] > mask_threshold (fp32, strict) else 0, and 0 outside the frame.
+ * The frame of slot s is frames[s / rows_per_frame] = (x0, y0, fw, fh) in rect coordinates
+ * (ceil(num_images*capacity / rows_per_frame) rows); frames NULL: frame f is image f at (0, 0), which
+ * needs rows_per_frame >= capacity. paste_boxes are xyxy in frame coordinates, mask_probs
+ * [num_images*capacity, M, M] by slot. masks_out receives h*w bytes per crop, packed in crop order at
+ * offsets[j] / channels (mb_crop_gather need not run). If totals[1] / channels exceeds
+ * masks_capacity_bytes nothing is written and totals[3] is set to 1, else totals[3] = 0.
+ * M + 2*padding <= 64. */
+int mb_crop_masks(const mb_crop_params* params_host, const float* mask_probs, const float* paste_boxes,
+                  int32_t mask_side, int32_t padding, const int32_t* frames, int32_t rows_per_frame,
+                  float mask_threshold, const int32_t* rects, const int32_t* src, const int64_t* offsets,
+                  int64_t* totals, uint8_t* masks_out, int64_t masks_capacity_bytes, mb_stream_t stream);
 /* maskrcnn_inference (tv:models/detection/roi_heads.py:56-82): mask_logits [R, C, M, M], labels [R] int64 ->
  * out [R, 1, M, M] = sigmoid(mask_logits[r, labels[r]]). Labels outside [0, C) are the caller's error. */
 int mb_mask_prob(const float* mask_logits, const int64_t* labels, int64_t num_masks, int32_t num_classes,

@@ -78,12 +78,20 @@ def crop_objects(tasks, output_dir, wsl2, api):
 @click.option('--model', type=str, prompt='Name of folder containing model')
 @click.option('--threshold', type=float, default=0.5, help='Detection threshold')
 @click.option('--batch-size', type=int, default=2)
-def infer_object_detector_directory(input_dir, output_dir, model_dir, model, threshold, batch_size):
+@click.option('--mask-dir', type=str, default=None,
+              help='Also write each crop\'s instance mask (Mask R-CNN models) as a PNG under this folder, same relative path')
+def infer_object_detector_directory(input_dir, output_dir, model_dir, model, threshold, batch_size, mask_dir):
     model_path = os.path.join(model_dir, model, "model.pt")
     labels = read_labels(os.path.join(model_dir, model, "labels.txt"))
-    project = infer_directory_fn(input_dir, model_path, labels, threshold, batch_size)
+    if mask_dir is None:
+        project = infer_directory_fn(input_dir, model_path, labels, threshold, batch_size)
+    else:
+        try:
+            project = infer_directory_fn(input_dir, model_path, labels, threshold, batch_size, with_masks=True)
+        except ValueError as e:
+            raise click.ClickException(str(e))
     Path(output_dir).mkdir(parents=True, exist_ok=True)
-    crop_objects_fn(project, output_dir, relative_to=input_dir)
+    crop_objects_fn(project, output_dir, relative_to=input_dir, mask_dir=mask_dir)
 
 
 if __name__ == "__main__":

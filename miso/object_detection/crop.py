@@ -24,7 +24,10 @@ def _imread(path: str) -> np.ndarray:
         return np.array(img)                       # copy: PIL-backed arrays are read-only
 
 
-def crop_objects(project: Project, output_dir: str, relative_to=None):
+def crop_objects(project: Project, output_dir: str, relative_to=None, mask_dir=None):
+    """Crops of every annotation under output_dir/<sub-folders>/<label>/. With mask_dir, each annotation's instance mask
+    (`mask`, set by inference with_masks=True) is written as well, as a PNG (mode L, 0 / 255) with the crop's relative
+    path and file name under mask_dir — a separate tree, so classifiers trained on the crop folders never see it."""
     from PIL import Image
     from miso_b200 import detection
     os.makedirs(output_dir, exist_ok=True)
@@ -71,6 +74,13 @@ def crop_objects(project: Project, output_dir: str, relative_to=None):
             filename = f"{path.stem}_{s[0]:.0f}_{s[1]:.0f}_{s[2]:.0f}_{s[3]:.0f}{path.suffix}"
             if crop.size:
                 pending.append(pool.submit(save, crop, os.path.join(str(label_path), filename)))
+                if mask_dir is not None and getattr(box, "mask", None) is not None:
+                    if box.mask.shape != crop.shape[:2]:
+                        raise ValueError(f"crop_objects: mask {box.mask.shape} of {filename} differs from its crop "
+                                         f"{crop.shape[:2]} (annotation changed after inference?)")
+                    mask_path = Path(mask_dir) / label_path.relative_to(output_path)
+                    mask_path.mkdir(parents=True, exist_ok=True)
+                    pending.append(pool.submit(save, box.mask, str(mask_path / Path(filename).with_suffix(".png"))))
     for f in pending:
         f.result()                      # re-raise encoder / file-system errors
     pool.shutdown()

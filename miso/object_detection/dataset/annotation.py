@@ -7,10 +7,11 @@ import numpy as np
 
 
 class RectangleAnnotation:
-    def __init__(self, x, y, width, height, label, score=1.0, annotator=None, validator=None, uid=None):
+    def __init__(self, x, y, width, height, label, score=1.0, annotator=None, validator=None, uid=None, mask=None):
         self.x, self.y, self.width, self.height = x, y, width, height
         self.label, self.score = label, score
         self.annotator, self.validator, self.uid = annotator, validator, uid
+        self.mask = mask        # np.uint8 [h, w] instance mask (0 / 255) over the crop rectangle, or None
 
     @property
     def bounds(self):

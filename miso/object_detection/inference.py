@@ -39,12 +39,16 @@ def read_image(path) -> np.ndarray:
 
 
 def _annotate(model, images_meta: List[ImageMetadata], model_labels, threshold, batch_size, project_out: Project,
-              num_workers: int = 4):
+              num_workers: int = 4, with_masks: bool = False):
     """One pass over the images: decode (a pool of `num_workers` threads reads and decodes the next batches while the
     GPU works — the reference uses a DataLoader with 4 workers, ref:miso/object_detection/inference.py:102-109),
-    patched model, score filter + bounds on the device, annotations."""
+    patched model, score filter + bounds on the device, annotations. with_masks (Mask R-CNN): every annotation also
+    gets `mask`, its detection's instance mask over the crop rectangle (np.uint8 [h, w], 0 / 255), cut on the device
+    by the same filter_and_crop call."""
     from concurrent.futures import ThreadPoolExecutor
     from miso_b200 import detection
+    if with_masks and getattr(model.roi_heads, "mask_predictor", None) is None:
+        raise ValueError("instance masks need a Mask R-CNN model; this model has no mask head")
     starts = list(range(0, len(images_meta), batch_size))
     with torch.inference_mode(), ThreadPoolExecutor(max_workers=max(1, num_workers)) as pool:
         window = max(2 * batch_size, num_workers)           # images being read / decoded ahead of the GPU
@@ -58,8 +62,12 @@ def _annotate(model, images_meta: List[ImageMetadata], model_labels, threshold, 
             dev_u8 = [torch.from_numpy(np.ascontiguousarray(a).copy() if not a.flags.writeable else a).cuda() for a in arrays]
             if getattr(model, "_miso_b200_patched", False) and all(a.dim() == 3 and a.shape[2] == 3 for a in dev_u8):
                 from miso_b200.patch import forward_uint8
-                results = forward_uint8(model, dev_u8)       # ToTensor + model.transform fused into one kernel
+                # ToTensor + model.transform fused into one kernel; Mask R-CNN masks stay 28x28 probabilities (a full-image
+                # paste per detection would be thrown away, or cut to the crop rectangles below)
+                results = forward_uint8(model, dev_u8, paste_masks=False)
             else:
+                if with_masks:
+                    raise ValueError("instance masks need a model patched by miso_b200.patch.patch_model and RGB images")
                 images_cuda = [a.permute(2, 0, 1).to(torch.float32) / 255 for a in dev_u8]       # ToTensor
                 results = model(images_cuda)
             pad = torch.nn.utils.rnn.pad_sequence
@@ -73,22 +81,25 @@ def _annotate(model, images_meta: List[ImageMetadata], model_labels, threshold, 
                     project_out.add_image(m)
                 continue
             counts = torch.tensor(counts_host, dtype=torch.int32, device="cuda")
-            out = detection.filter_and_crop(dev_u8, boxes.contiguous(), scores.contiguous(), counts, threshold, capacity_bytes=0)
+            probs = pad([r["mask_probs"][:, 0] for r in results], batch_first=True) if with_masks else None
+            out = detection.filter_and_crop(dev_u8, boxes.contiguous(), scores.contiguous(), counts, threshold, capacity_bytes=0,
+                                            mask_probs=probs)
             kept = int(out.totals[0])
+            masks = out.masks_to_host() if with_masks else [None] * kept
             xywh = out.xywh[:kept].cpu().numpy()
             src = out.src[:kept].cpu().numpy()
             labels = labels_d.cpu().numpy()
             for j in range(kept):
                 k, d = int(src[j]) // cap, int(src[j]) % cap
                 x, y, w, h = xywh[j]
-                metas[k].boxes.append(RectangleAnnotation(x, y, w, h, model_labels[int(labels[k, d]) - 1]))
+                metas[k].boxes.append(RectangleAnnotation(x, y, w, h, model_labels[int(labels[k, d]) - 1], mask=masks[j]))
             for m in metas:
                 project_out.add_image(m)
     return project_out
 
 
 def infer(project: Project, model_path: str, model_labels: List[str] = None, threshold: float = 0.5, batch_size=2,
-          nv: bool = False):
+          nv: bool = False, with_masks: bool = False):
     if nv:
         model_labels = [label + "_NV" for label in model_labels]
     for label in model_labels:
@@ -99,10 +110,11 @@ def infer(project: Project, model_path: str, model_labels: List[str] = None, thr
     out = Project()
     for label in model_labels:
         out.add_label(None, label, None)
-    return _annotate(model, list(project.image_dict.values()), model_labels, threshold, batch_size, out)
+    return _annotate(model, list(project.image_dict.values()), model_labels, threshold, batch_size, out, with_masks=with_masks)
 
 
-def infer_directory(input_dir: str, model_path: str, model_labels: List[str] = None, threshold: float = 0.5, batch_size=2):
+def infer_directory(input_dir: str, model_path: str, model_labels: List[str] = None, threshold: float = 0.5, batch_size=2,
+                    with_masks: bool = False):
     p = Path(input_dir)
     if not p.exists():
         raise ValueError(f"Directory does not exist: {input_dir}")
@@ -112,4 +124,4 @@ def infer_directory(input_dir: str, model_path: str, model_labels: List[str] = N
     out = Project()
     for label in model_labels:
         out.add_label(None, label, None)
-    return _annotate(model, metas, model_labels, threshold, batch_size, out)
+    return _annotate(model, metas, model_labels, threshold, batch_size, out, with_masks=with_masks)

@@ -113,6 +113,7 @@ SIGNATURES = {
     "mb_roi_align_backward": (C.c_int, [_p, _p, _i64, _f32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _p, _p]),
     "mb_paste_masks": (C.c_int, [_p, _p, _i64, _i32, _i32, _i32, _i32, _p, _p]),
     "mb_mask_prob": (C.c_int, [_p, _p, _i64, _i32, _i32, _p, _p]),
+    "mb_crop_masks": (C.c_int, [C.POINTER(CropParams), _p, _p, _i32, _i32, _p, _i32, _f32, _p, _p, _p, _p, _p, _i64, _p]),
     "mb_image_transform": (C.c_int, [C.POINTER(TransformParams), _p, _p]),
 }
 

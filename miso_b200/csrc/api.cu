@@ -6,7 +6,7 @@ extern "C" int mb_abi_version(void) { return MB_ABI_VERSION; }
 extern "C" const char* mb_build_info(void) {
     return "libmisob200 sm_100a cuda " __DATE__
            ";kernels="
-           "k_box_convert,k_box_decode,k_box_iou,k_box_max,k_clip_boxes,k_crop_gather,k_crop_plan,"
+           "k_box_convert,k_box_decode,k_box_iou,k_box_max,k_clip_boxes,k_crop_gather,k_crop_masks,k_crop_plan,"
            "k_crop_plan_chunks,k_det_candidates,k_det_finalize,k_det_init,k_emit_single,k_emit_sorted,"
            "k_grid_anchors,k_group_hist,k_image_transform,k_kept_bucket,k_mask_prob,k_match_best,k_match_finish,"
            "k_mosaic_pack,k_mosaic_unpack,k_nchw_to_nhwc,k_nms_fixpoint,k_nms_mask,k_nms_sweep,k_nms_sweep_small,"

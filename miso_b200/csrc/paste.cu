@@ -13,6 +13,11 @@
 // 0, lambda = clamp(src - floor(src), 0, 1), value = fma(fma(v00, wx0, v01*wx1), wy0,
 // fma(v10, wx0, v11*wx1) * wy1)): bit-identical to the reference for outputs of >= ~1600 pixels,
 // within 1 ulp below (the reference's own small-output loop contracts differently).
+//
+// k_crop_masks (mb_crop_masks) is the same paste evaluated only at the pixels of each crop rectangle of mb_crop_plan and
+// thresholded to 0 / 255 bytes: the per-crop instance masks without the [R, H, W] fp32 frame.
+#include <algorithm>
+
 #include "common.cuh"
 
 namespace mb {
@@ -52,6 +57,15 @@ __device__ __forceinline__ void paste_tap(float scale, int d, int padded, int& i
     i1 = i0 + (i0 < padded - 1 ? 1 : 0);
 }
 
+// ATen's bilinear value (UpSampleKernel.cpp, as compiled with FMA contraction) from two padded mask rows; every kernel
+// that produces a pasted mask value calls this, so a pixel has the same bits in all of them
+__device__ __forceinline__ float paste_value(const float* r0, const float* r1, int x0, int x1, float wx0, float wx1,
+                                             float wy0, float wy1) {
+    const float t0 = fmaf(r0[x0], wx0, __fmul_rn(r0[x1], wx1));
+    const float t1 = fmaf(r1[x0], wx0, __fmul_rn(r1[x1], wx1));
+    return fmaf(t0, wy0, __fmul_rn(t1, wy1));
+}
+
 __global__ void __launch_bounds__(kPasteThreads) k_paste_masks(const float* __restrict__ masks, const float4* __restrict__ boxes,
                                                                int M, int padding, float mask_scale, int H, int W,
                                                                float* __restrict__ out) {
@@ -87,9 +101,7 @@ __global__ void __launch_bounds__(kPasteThreads) k_paste_masks(const float* __re
                     if (x >= ax.lo && x < ax.hi) {
                         int x0, x1; float wx0, wx1;
                         paste_tap(ax.scale, x - ax.org, P, x0, x1, wx0, wx1);
-                        const float t0 = fmaf(r0[x0], wx0, __fmul_rn(r0[x1], wx1));
-                        const float t1 = fmaf(r1[x0], wx0, __fmul_rn(r1[x1], wx1));
-                        v[j] = fmaf(t0, wy0, __fmul_rn(t1, wy1));
+                        v[j] = paste_value(r0, r1, x0, x1, wx0, wx1, wy0, wy1);
                     }
                 }
             }
@@ -98,6 +110,103 @@ __global__ void __launch_bounds__(kPasteThreads) k_paste_masks(const float* __re
             } else {
 #pragma unroll
                 for (int j = 0; j < 4; ++j) if (x4 + j < W) row[x4 + j] = v[j];
+            }
+        }
+    }
+}
+
+// Instance masks cut to the crop rectangles of mb_crop_plan: crop j (slot s = src[j], rectangle rc) gets
+// (paste of mask s into its frame)[rc] > thr as 0 / 255 bytes, 0 where rc leaves the frame — only the crop's pixels are
+// computed, never the frame. Work split of k_crop_gather: crops strided over blockIdx.x (the next crop's metadata
+// prefetched), rows over the warps; the padded mask sits in shared memory, the x taps of the crop's columns are staged
+// next to it once per crop (kMaskCols columns per pass), the y taps once per row. Lanes write 4-byte words between the
+// row's unaligned ends.
+constexpr int kMaskThreads = 256;
+constexpr int kMaskCols = 1024;
+
+struct CropMaskDev {
+    int M, P, ch, rows_per_frame;
+    float mask_scale, thr;
+    int img_h[MB_MAX_IMAGES], img_w[MB_MAX_IMAGES];     // frame f of a NULL frame table: image f at (0, 0)
+};
+
+__global__ void __launch_bounds__(kMaskThreads) k_crop_masks(const CropMaskDev d, const float* __restrict__ probs,
+                                                             const float4* __restrict__ boxes, const int4* __restrict__ frames,
+                                                             const int4* __restrict__ rects, const int* __restrict__ src,
+                                                             const long long* __restrict__ offsets, long long* __restrict__ totals,
+                                                             unsigned char* __restrict__ out, long long capacity) {
+    __shared__ float sm[kPasteMaxSide * kPasteMaxSide];
+    __shared__ int2 taps[kMaskCols];       // (x0, bits of lambda1); x0 = -1: inside the frame, outside the paste box; -2: outside the frame
+    const long long ncrops = totals[0];
+    const bool overflow = totals[1] / d.ch > capacity;
+    if (blockIdx.x == 0 && threadIdx.x == 0) totals[3] = overflow ? 1 : 0;      // caller re-runs with totals[1] / ch bytes
+    if (overflow) return;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    constexpr int nwarps = kMaskThreads / 32;
+    const int M = d.M, P = d.P, pad = (P - M) / 2;
+    int4 rc_next = make_int4(0, 0, 0, 0);
+    int src_next = 0;
+    long long off_next = 0;
+    if ((long long)blockIdx.x < ncrops) { rc_next = rects[blockIdx.x]; src_next = src[blockIdx.x]; off_next = offsets[blockIdx.x]; }
+    for (long long j = blockIdx.x; j < ncrops; j += gridDim.x) {
+        const int4 rc = rc_next;
+        const int s = src_next;
+        unsigned char* dst = out + off_next / d.ch;         // every crop holds h * w * ch bytes
+        const long long jn = j + gridDim.x;
+        if (jn < ncrops) { rc_next = rects[jn]; src_next = src[jn]; off_next = offsets[jn]; }
+        if (rc.z == 0 || rc.w == 0) continue;
+        const int f = s / d.rows_per_frame;
+        const int4 fr = frames ? frames[f] : make_int4(0, 0, d.img_w[f], d.img_h[f]);      // (x0, y0, w, h)
+        __syncthreads();                                     // the previous crop's mask and taps are no longer read
+        const float* mk = probs + (size_t)s * M * M;
+        for (int i = tid; i < P * P; i += kMaskThreads) {    // F.pad(mask, (padding,) * 4)
+            const int y = i / P - pad, x = i % P - pad;
+            sm[i] = (y >= 0 && y < M && x >= 0 && x < M) ? mk[y * M + x] : 0.f;
+        }
+        const float4 b = boxes[s];
+        PasteAxis ax, ay;
+        paste_axis(b.x, b.z, d.mask_scale, P, fr.z, ax);
+        paste_axis(b.y, b.w, d.mask_scale, P, fr.w, ay);
+        for (int c0 = 0; c0 < rc.z; c0 += kMaskCols) {
+            const int cn = min(kMaskCols, rc.z - c0);
+            if (c0 > 0) __syncthreads();
+            for (int c = tid; c < cn; c += kMaskThreads) {
+                const int fx = rc.x + c0 + c - fr.x;
+                int2 t = make_int2(fx >= 0 && fx < fr.z ? -1 : -2, 0);
+                if (fx >= ax.lo && fx < ax.hi) {
+                    int x0, x1; float w0, w1;
+                    paste_tap(ax.scale, fx - ax.org, P, x0, x1, w0, w1);
+                    t = make_int2(x0, __float_as_int(w1));
+                }
+                taps[c] = t;
+            }
+            __syncthreads();
+            for (int r = warp; r < rc.w; r += nwarps) {
+                const int fy = rc.y + r - fr.y;
+                const bool in_frame = fy >= 0 && fy < fr.w;
+                const bool live = fy >= ay.lo && fy < ay.hi;     // [lo, hi) lies inside the frame
+                int y0 = 0, y1 = 0; float wy0 = 0.f, wy1 = 0.f;
+                if (live) paste_tap(ay.scale, fy - ay.org, P, y0, y1, wy0, wy1);
+                const float* r0 = sm + y0 * P; const float* r1 = sm + y1 * P;
+                auto px = [&](int c) -> unsigned {
+                    const int2 t = taps[c];
+                    if (!in_frame || t.x == -2) return 0u;
+                    float v = 0.f;                               // the paste's zero image outside the box
+                    if (live && t.x >= 0) {
+                        const float w1 = __int_as_float(t.y);
+                        v = paste_value(r0, r1, t.x, t.x + (t.x < P - 1 ? 1 : 0), __fsub_rn(1.0f, w1), w1, wy0, wy1);
+                    }
+                    return v > d.thr ? 255u : 0u;
+                };
+                unsigned char* orow = dst + (size_t)r * rc.z + c0;
+                const int head = min(cn, (int)((4u - ((unsigned)reinterpret_cast<uintptr_t>(orow) & 3u)) & 3u));
+                const int nw = (cn - head) >> 2, tail = head + 4 * nw;
+                if (lane < head) orow[lane] = (unsigned char)px(lane);
+                for (int i = lane; i < nw; i += 32) {
+                    const int c = head + 4 * i;
+                    *reinterpret_cast<unsigned*>(orow + c) = px(c) | (px(c + 1) << 8) | (px(c + 2) << 16) | (px(c + 3) << 24);
+                }
+                if (lane < cn - tail) orow[tail + lane] = (unsigned char)px(tail + lane);
             }
         }
     }
@@ -144,6 +253,34 @@ extern "C" int mb_paste_masks(const float* masks, const float* boxes, int64_t nu
     dim3 grid((im_h + mb::kPasteRows - 1) / mb::kPasteRows, (unsigned)num_masks);
     mb::k_paste_masks<<<grid, mb::kPasteThreads, 0, (cudaStream_t)stream>>>(masks, reinterpret_cast<const float4*>(boxes), mask_side,
                                                                            padding, mask_scale, im_h, im_w, out);
+    MB_LAUNCH_CHECK();
+    return MB_OK;
+}
+
+extern "C" int mb_crop_masks(const mb_crop_params* p, const float* mask_probs, const float* paste_boxes, int32_t mask_side,
+                             int32_t padding, const int32_t* frames, int32_t rows_per_frame, float mask_threshold,
+                             const int32_t* rects, const int32_t* src, const int64_t* offsets, int64_t* totals,
+                             uint8_t* masks_out, int64_t masks_capacity_bytes, mb_stream_t stream) {
+    if (!p || mask_side < 1 || padding < 0 || rows_per_frame < 1 || masks_capacity_bytes < 0) return MB_ERR_INVALID_ARG;
+    if (p->num_images < 1 || p->num_images > MB_MAX_IMAGES || p->capacity < 1 || p->channels < 1) return MB_ERR_INVALID_ARG;
+    if (mask_side + 2 * padding > mb::kPasteMaxSide) return MB_ERR_UNSUPPORTED;
+    if (!mask_probs || !paste_boxes || !rects || !src || !offsets || !totals || (masks_capacity_bytes > 0 && !masks_out))
+        return MB_ERR_INVALID_ARG;
+    if (!frames && rows_per_frame < p->capacity) return MB_ERR_INVALID_ARG;        // frame f = image f needs f < num_images
+    mb::CropMaskDev d;
+    d.M = mask_side; d.P = mask_side + 2 * padding; d.ch = p->channels; d.rows_per_frame = rows_per_frame;
+    d.mask_scale = (float)((double)(mask_side + 2 * padding) / (double)mask_side);     // as mb_paste_masks
+    d.thr = mask_threshold;
+    for (int n = 0; n < MB_MAX_IMAGES; ++n) {
+        const bool used = n < p->num_images;
+        if (used && (p->image_h[n] < 0 || p->image_w[n] < 0)) return MB_ERR_INVALID_ARG;
+        d.img_h[n] = used ? p->image_h[n] : 0; d.img_w[n] = used ? p->image_w[n] : 0;
+    }
+    const long long slots = (long long)p->num_images * p->capacity;
+    const int grid = (int)std::min<long long>(std::max<long long>(slots, 1), (long long)mb::num_sms() * 8);
+    mb::k_crop_masks<<<grid, mb::kMaskThreads, 0, (cudaStream_t)stream>>>(
+        d, mask_probs, reinterpret_cast<const float4*>(paste_boxes), reinterpret_cast<const int4*>(frames),
+        reinterpret_cast<const int4*>(rects), src, (const long long*)offsets, (long long*)totals, masks_out, masks_capacity_bytes);
     MB_LAUNCH_CHECK();
     return MB_OK;
 }

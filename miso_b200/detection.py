@@ -214,12 +214,13 @@ def postprocess_detections(class_logits: Tensor, box_regression: Tensor, proposa
 # ------------------------------------------------------------------------------------------
 @dataclass
 class CropOutput:
-    totals: Tensor     # [4] int64: number of crops, total bytes, overflow flag
+    totals: Tensor     # [4] int64: number of crops, total bytes, pixel overflow flag, mask overflow flag
     rects: Tensor      # [N*cap, 4] int32 (x_begin, y_begin, width, height)
     xywh: Tensor       # [N*cap, 4] fp32 annotation bounds (x, y, w, h)
     src: Tensor        # [N*cap] int32: n*cap + detection index
     offsets: Tensor    # [N*cap+1] int64 byte offsets into `pixels`
     pixels: Tensor     # [capacity] uint8 packed crops (HWC each)
+    masks: Optional[Tensor] = None     # uint8 packed h*w masks (0 / 255) of the crops at offsets // channels
 
     def to_host(self, channels: int):
         """One device->host transfer; returns per-crop (image index, detection index, xywh, array)."""
@@ -237,13 +238,34 @@ class CropOutput:
             out.append((int(src[j]) // cap, int(src[j]) % cap, xywh[j], a))
         return out
 
+    def masks_to_host(self) -> List:
+        """The crops' masks as np.uint8 [h, w] arrays in crop order (one device->host transfer of the packed bytes)."""
+        if self.masks is None:
+            raise MisoB200Error("no masks: filter_and_crop ran without mask_probs")
+        tot = self.totals.tolist()
+        if tot[3]:
+            raise MisoB200Error(f"mask buffer too small: {tot[1] // self._ch} bytes needed")
+        k = tot[0]
+        rects = self.rects[:k].cpu().numpy()
+        offs = self.offsets[:k + 1].cpu().numpy() // self._ch
+        buf = self.masks[:tot[1] // self._ch].cpu().numpy()
+        return [buf[offs[j]:offs[j + 1]].reshape(rects[j][3], rects[j][2]) for j in range(k)]
+
     _n: int = 1
+    _ch: int = 1
 
 
 def filter_and_crop(images: Sequence[Tensor], det_boxes: Tensor, det_scores: Tensor, det_counts: Tensor,
-                    threshold: float, capacity_bytes: Optional[int] = None, boxes_are_xywh: bool = False) -> CropOutput:
+                    threshold: float, capacity_bytes: Optional[int] = None, boxes_are_xywh: bool = False,
+                    mask_probs: Optional[Tensor] = None, paste_boxes: Optional[Tensor] = None, mask_threshold: float = 0.5,
+                    mask_capacity_bytes: Optional[int] = None) -> CropOutput:
     """images[n]: uint8 [H, W, C] or [H, W] on the device (the ORIGINAL image pixels, as
-    skimage.io.imread returns them); det_* as produced by postprocess_detections."""
+    skimage.io.imread returns them); det_* as produced by postprocess_detections.
+
+    mask_probs ([N, cap, M, M] or [N*cap, 1, M, M], Mask R-CNN's per-detection probabilities) adds each crop's instance
+    mask (mb_crop_masks): paste_masks_in_image of the detection's mask into its image at paste_boxes (default
+    det_boxes, xyxy), cut to the crop rectangle, 255 where > mask_threshold else 0. capacity_bytes = 0 skips the pixel
+    gather; mask_capacity_bytes None sizes the mask buffer exactly (one host sync)."""
     lib = _lib.load()
     n, cap = det_boxes.shape[0], det_boxes.shape[1]
     if len(images) != n:
@@ -279,6 +301,19 @@ def filter_and_crop(images: Sequence[Tensor], det_boxes: Tensor, det_scores: Ten
     pixels = torch.empty((max(int(capacity_bytes), 1),), dtype=torch.uint8, device=dev)
     _lib.check(lib.mb_crop_gather(C.byref(p), _ptr(rects), _ptr(src), _ptr(offsets), _ptr(totals), _ptr(pixels),
                                   int(capacity_bytes), st), "mb_crop_gather")
-    out = CropOutput(totals, rects, xywh, src, offsets, pixels)
-    out._n = n
+    masks = None
+    if mask_probs is not None:
+        m = int(mask_probs.shape[-1])
+        mp = _f32c(mask_probs)
+        torch._assert(mp.numel() == n * cap * m * m and mp.shape[-2] == m, "mask_probs must be [N, cap, M, M] or [N*cap, 1, M, M]")
+        pb = b if paste_boxes is None else _f32c(paste_boxes)
+        torch._assert(pb.numel() == n * cap * 4, "paste_boxes must be [N, cap, 4]")
+        if mask_capacity_bytes is None:
+            mask_capacity_bytes = int(totals[1].item()) // ch
+        masks = torch.empty((max(int(mask_capacity_bytes), 1),), dtype=torch.uint8, device=dev)
+        _lib.check(lib.mb_crop_masks(C.byref(p), _ptr(mp), _ptr(pb), m, 1, None, cap, float(mask_threshold), _ptr(rects),
+                                     _ptr(src), _ptr(offsets), _ptr(totals), _ptr(masks), int(mask_capacity_bytes), st),
+                   "mb_crop_masks")
+    out = CropOutput(totals, rects, xywh, src, offsets, pixels, masks)
+    out._n, out._ch = n, ch
     return out

@@ -202,6 +202,7 @@ class MosaicCrops:
         p.threshold = float(threshold)
         self.params = p
         self.band = None
+        self.mask_args = None
 
     def bind_band(self, band_u8: Tensor, band_y0: int) -> None:
         """band_u8: uint8 [band_h, W, C] — mosaic rows [band_y0, band_y0 + band_h). The crop kernels address the
@@ -214,6 +215,24 @@ class MosaicCrops:
         self.band, self.band_y0 = band_u8, int(band_y0)
         self.params.images[0] = band_u8.data_ptr() - self.band_y0 * band_u8.shape[1] * band_u8.shape[2]
 
+    def bind_masks(self, mask_probs: Tensor, paste_boxes: Tensor, frames: Tensor, rows_per_frame: int,
+                   mask_threshold: float = 0.5) -> None:
+        """Cut every crop's instance mask as well (mb_crop_masks after the gather, results()["masks"]). Row s of this
+        rank's block: mask_probs [rows, M, M] (maskrcnn_inference's output), paste_boxes [rows, 4] xyxy in the
+        coordinates of its frame, the tile it came from: frames[s // rows_per_frame] = (x0, y0, w, h) int32 in mosaic
+        coordinates. A crop's mask is the tile-sized paste_masks_in_image of its detection, cut to the crop rectangle
+        and thresholded (> mask_threshold: 255, else 0; 0 outside the tile)."""
+        m = int(mask_probs.shape[-1])
+        for t in (mask_probs, paste_boxes, frames):
+            torch._assert(t.is_cuda and t.is_contiguous(), "bind_masks: contiguous CUDA tensors expected")
+        torch._assert(mask_probs.dtype == torch.float32 and mask_probs.shape == (self.rows, m, m),
+                      "bind_masks: mask_probs must be fp32 [rows, M, M]")
+        torch._assert(paste_boxes.dtype == torch.float32 and paste_boxes.shape == (self.rows, 4), "bind_masks: paste_boxes must be fp32 [rows, 4]")
+        torch._assert(frames.dtype == torch.int32 and frames.dim() == 2 and frames.shape[1] == 4
+                      and frames.shape[0] * int(rows_per_frame) >= self.rows, "bind_masks: frames must be int32 [rows / rows_per_frame, 4]")
+        self.mask_args = (mask_probs, paste_boxes, frames, m, int(rows_per_frame), float(mask_threshold))
+        self.masks = torch.empty((max(self.capacity // self.params.channels, 1),), dtype=torch.uint8, device=mask_probs.device)
+
     def launch(self, gathered: Tensor, state: Tensor, row_lo: int) -> None:
         st = _cstream(gathered)
         _lib.check(self.lib.mb_seam_select(_p(gathered), _p(state), int(row_lo), self.rows, _p(self.boxes), _p(self.scores), st),
@@ -223,15 +242,27 @@ class MosaicCrops:
                                          _p(self.src), _p(self.offsets), _p(self.totals), st), "mb_crop_plan")
         _lib.check(self.lib.mb_crop_gather(cp, _p(self.rects), _p(self.src), _p(self.offsets), _p(self.totals),
                                            _p(self.pixels), self.capacity, st), "mb_crop_gather")
+        if self.mask_args is not None:
+            probs, boxes, frames, m, rpf, thr = self.mask_args
+            _lib.check(self.lib.mb_crop_masks(cp, _p(probs), _p(boxes), m, 1, _p(frames), rpf, thr, _p(self.rects), _p(self.src),
+                                              _p(self.offsets), _p(self.totals), _p(self.masks), self.masks.numel(), st),
+                       "mb_crop_masks")
 
     def results(self) -> Dict[str, Tensor]:
-        """One sync: this rank's surviving detections in row order and their crop bytes."""
+        """One sync: this rank's surviving detections in row order and their crop bytes; with bind_masks() also
+        "masks", the crops' h*w mask bytes packed at offsets // channels."""
         tot = self.totals.tolist()
         if tot[2]:
             raise MisoB200Error(f"mosaic crop buffer too small: {tot[1]} bytes needed, {self.capacity} available")
         k = tot[0]
-        return {"count": k, "bytes": tot[1], "rects": self.rects[:k], "xywh": self.xywh[:k], "src": self.src[:k],
-                "offsets": self.offsets[:k + 1], "pixels": self.pixels[:tot[1]]}
+        out = {"count": k, "bytes": tot[1], "rects": self.rects[:k], "xywh": self.xywh[:k], "src": self.src[:k],
+               "offsets": self.offsets[:k + 1], "pixels": self.pixels[:tot[1]]}
+        if self.mask_args is not None:
+            if tot[3]:
+                raise MisoB200Error(f"mosaic mask buffer too small: {tot[1] // self.params.channels} bytes needed, "
+                                    f"{self.masks.numel()} available")
+            out["masks"] = self.masks[:tot[1] // self.params.channels]
+        return out
 
 
 class MosaicPlan:
@@ -499,14 +530,19 @@ def by_score(gathered: Tensor, state: Tensor) -> Tensor:
 
 def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: int = 0, tile: int = 1024,
                  overlap: int = 128, threshold: float = 0.5, batch_size: int = 4, rank: int = 0, world: int = 1,
-                 group=None, crop_capacity_bytes: int = 256 << 20):
+                 group=None, crop_capacity_bytes: int = 256 << 20, masks: bool = False, mask_threshold: float = 0.5):
     """Detect on a large slide/mosaic image (config 5) with a (patched) torchvision detection model: this rank runs
     its contiguous share of tiles, the per-rank detection blocks are exchanged with one all-gather, the sparse seam
     NMS runs on every rank (replicated, deterministic) and each rank cuts the crops of its own tiles' survivors.
 
     band_u8: uint8 [band_h, W, C] on the device = mosaic rows [band_y0, band_y0 + band_h) — the pixel band this
     rank's tiles cover (rank_band()); with world == 1 simply the whole mosaic. Returns a dict: gathered [rows, 6]
-    (mosaic coordinates), state [rows] (1 = kept), and this rank's crops (MosaicCrops.results())."""
+    (mosaic coordinates), state [rows] (1 = kept), and this rank's crops (MosaicCrops.results()).
+    masks=True (Mask R-CNN): crops["masks"] holds every crop's instance mask, its detection's mask pasted into the
+    tile it came from, cut to the crop rectangle, > mask_threshold -> 255 (MosaicCrops.bind_masks)."""
+    has_mask = getattr(model.roi_heads, "mask_predictor", None) is not None
+    if masks and not has_mask:
+        raise MisoB200Error("infer_mosaic(masks=True): the model has no mask head (Mask R-CNN needed)")
     dev = band_u8.device
     h, w = int(mosaic_hw[0]), int(mosaic_hw[1])
     grid = tile_grid(h, w, tile, overlap)
@@ -517,19 +553,28 @@ def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: in
     scores = torch.zeros((max(len(mine), 1), dpi), dtype=torch.float32, device=dev)
     labels = torch.zeros((max(len(mine), 1), dpi), dtype=torch.int64, device=dev)
     counts = torch.zeros((max(len(mine), 1),), dtype=torch.int32, device=dev)
+    probs = None
     with torch.inference_mode():
         for i0 in range(0, len(mine), batch_size):
             idx = mine[i0:i0 + batch_size]
             tiles = [band_u8[grid[t][0] - band_y0:grid[t][0] - band_y0 + tile, grid[t][1]:grid[t][1] + tile] for t in idx]
             if getattr(model, "_miso_b200_patched", False) and band_u8.shape[2] <= 4:
                 from .patch import forward_uint8
-                res = forward_uint8(model, tiles)        # ToTensor + normalize + resize + batch in one kernel
+                # ToTensor + normalize + resize + batch in one kernel; no full-tile mask paste (nobody reads it)
+                res = forward_uint8(model, tiles, paste_masks=False)
             else:
                 res = model([t.permute(2, 0, 1).to(torch.float32) / 255 for t in tiles])
             for j, r in enumerate(res):
                 k = int(r["boxes"].shape[0])
                 boxes[i0 + j, :k], scores[i0 + j, :k], labels[i0 + j, :k] = r["boxes"], r["scores"], r["labels"]
                 counts[i0 + j] = k
+                if masks:
+                    if "mask_probs" not in r:
+                        raise MisoB200Error("infer_mosaic(masks=True) needs a model patched by miso_b200.patch.patch_model")
+                    if probs is None:
+                        m = int(r["mask_probs"].shape[-1])
+                        probs = torch.zeros((tmax * dpi, m, m), dtype=torch.float32, device=dev)
+                    probs[(i0 + j) * dpi:(i0 + j) * dpi + k] = r["mask_probs"][:, 0]
     origins = torch.tensor([[float(grid[t][0]), float(grid[t][1])] for t in mine] or [[0.0, 0.0]], dtype=torch.float32,
                            device=dev).reshape(-1, 2)
     block = torch.zeros((tmax * dpi, 6), dtype=torch.float32, device=dev)
@@ -542,6 +587,18 @@ def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: in
     state = seam.launch(gathered, float(model.roi_heads.nms_thresh))
     crops = MosaicCrops(tmax * dpi, (h, w), int(band_u8.shape[2]), threshold, crop_capacity_bytes, dev)
     crops.bind_band(band_u8, band_y0)
+    if masks and probs is not None:
+        # frame of own row s: the tile it came from (boxes are tile-local, which is what the paste wants)
+        frames = torch.zeros((tmax, 4), dtype=torch.int32)
+        for i, t in enumerate(mine):
+            y, x = grid[t]
+            frames[i] = torch.tensor([x, y, min(tile, w - x), min(tile, h - y)], dtype=torch.int32)
+        paste_boxes = torch.zeros((tmax * dpi, 4), dtype=torch.float32, device=dev)
+        paste_boxes[:len(mine) * dpi] = boxes[:len(mine)].reshape(-1, 4)
+        crops.bind_masks(probs, paste_boxes, frames.to(dev), dpi, mask_threshold)
     crops.launch(gathered, state, rank * tmax * dpi)
     seam.check()
-    return {"gathered": gathered, "state": state, "crops": crops.results()}
+    res = crops.results()
+    if masks and probs is None:                    # no own tiles: no crops
+        res["masks"] = torch.empty((0,), dtype=torch.uint8, device=dev)
+    return {"gathered": gathered, "state": state, "crops": res}

@@ -108,10 +108,13 @@ def _transform_postprocess(self, result, image_shapes, original_image_sizes):
     return result
 
 
-def forward_uint8(model, images_u8: List[Tensor]):
+def forward_uint8(model, images_u8: List[Tensor], paste_masks: bool = True):
     """GeneralizedRCNN.forward (tv:models/detection/generalized_rcnn.py:47-119, eval branch) for uint8 HWC CUDA
     images: ToTensor + normalize + resize + batch run as one kernel (ops.transform_images) instead of the
-    reference's per-image tensor operations; everything downstream is the model's own (patched) code."""
+    reference's per-image tensor operations; everything downstream is the model's own (patched) code.
+    paste_masks=False (Mask R-CNN): each result carries `mask_probs` [k, 1, M, M] (maskrcnn_inference's output) instead
+    of the full-image `masks`, and no [k, 1, H, W] paste runs — for callers that cut the masks to crops
+    (detection.filter_and_crop, mosaic.MosaicCrops.bind_masks)."""
     from torchvision.models.detection.image_list import ImageList
     tr = model.transform
     original_image_sizes = [(int(im.shape[0]), int(im.shape[1])) for im in images_u8]
@@ -128,6 +131,10 @@ def forward_uint8(model, images_u8: List[Tensor]):
         features = {"0": features}
     proposals, _ = model.rpn(images, features)
     detections, _ = model.roi_heads(features, proposals, images.image_sizes)
+    if not paste_masks:
+        for d in detections:
+            if "masks" in d:
+                d["mask_probs"] = d.pop("masks")         # transform.postprocess pastes only a "masks" entry
     return tr.postprocess(detections, images.image_sizes, original_image_sizes)
 
 
