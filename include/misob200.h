@@ -308,6 +308,33 @@ int mb_crop_masks(const mb_crop_params* params_host, const float* mask_probs, co
                   int32_t mask_side, int32_t padding, const int32_t* frames, int32_t rows_per_frame,
                   float mask_threshold, const int32_t* rects, const int32_t* src, const int64_t* offsets,
                   int64_t* totals, uint8_t* masks_out, int64_t masks_capacity_bytes, mb_stream_t stream);
+/* Per-crop region measurements from the masks of mb_crop_masks (skimage.measure.regionprops of (mask > 0) with
+ * one label). The region of crop j is the set of non-zero bytes of its h*w mask at masks + offsets[j] / channels;
+ * (r, c) are crop-local row / column, rect (x, y, w, h). Exact int64 sums over the set pixels: A = sum 1,
+ * S_r, S_c, S_rr, S_cc, S_rc (sums of r, c, r*r, c*c, r*c), P_k = sum of pixel byte k, read from
+ * params.images[src[j] / capacity] at the rect (the pixel gather need not have run). out receives
+ * MB_MORPH_FIELDS fp64 per crop, at row j of [num_images*capacity, MB_MORPH_FIELDS], all 0 when A = 0:
+ *   0 area = A
+ *   1 perimeter (4-neighbourhood): E = mask with every pixel cleared that has a 4-neighbour outside it,
+ *     B = mask and not E; per p in B, code = 1 + 2 * (4-neighbours in B) + 10 * (diagonal neighbours in B);
+ *     n1 = #codes in {5,7,15,17,25,27}, n2 = #{21,33}, n3 = #{13,23};
+ *     perimeter = (n1 + sqrt2 * n2) + ((1 + sqrt2) / 2) * n3
+ *   2, 3 centroid_x = x + S_c / A, centroid_y = y + S_r / A
+ *   4, 5 major / minor_axis_length = 4 sqrt(l1), 4 sqrt(l2) with a = u_cc, b = -u_rc, c = u_rr,
+ *     u_rr = (A S_rr - S_r^2) / (A * A) (numerator exact in 128 bits, converted once; A * A in fp64), likewise
+ *     u_cc, u_rc = (A S_rc - S_r S_c) / (A * A); l1,2 = ((a + c) +- sqrt((a - c)^2 + 4 (b * b))) / 2, clipped at 0
+ *   6 orientation = a == c ? (b < 0 ? -pi/4 : pi/4) : atan2(-2 b, c - a) / 2
+ *   7 eccentricity = l1 == 0 ? 0 : sqrt(1 - l2 / l1)
+ *   8 equivalent_diameter = sqrt(4 A / pi)
+ *   9..12 mean_intensity_k = P_k / A for k < channels, else 0
+ * The count is totals[0] (device); if totals[3] (mask overflow) is set nothing is written. workspace: at least
+ * mb_mask_morphology_workspace_bytes(params) = 128 * num_images * capacity bytes (zeroed by the call).
+ * MB_ERR_UNSUPPORTED for channels > 4 or an image side > 32768 (which keeps every int64 sum exact). */
+#define MB_MORPH_FIELDS 13
+size_t mb_mask_morphology_workspace_bytes(const mb_crop_params* params_host);
+int mb_mask_morphology(const mb_crop_params* params_host, const uint8_t* masks, const int32_t* rects,
+                       const int32_t* src, const int64_t* offsets, const int64_t* totals, void* workspace,
+                       size_t workspace_bytes, double* out, mb_stream_t stream);
 /* maskrcnn_inference (tv:models/detection/roi_heads.py:56-82): mask_logits [R, C, M, M], labels [R] int64 ->
  * out [R, 1, M, M] = sigmoid(mask_logits[r, labels[r]]). Labels outside [0, C) are the caller's error. */
 int mb_mask_prob(const float* mask_logits, const int64_t* labels, int64_t num_masks, int32_t num_classes,

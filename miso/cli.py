@@ -80,18 +80,22 @@ def crop_objects(tasks, output_dir, wsl2, api):
 @click.option('--batch-size', type=int, default=2)
 @click.option('--mask-dir', type=str, default=None,
               help='Also write each crop\'s instance mask (Mask R-CNN models) as a PNG under this folder, same relative path')
-def infer_object_detector_directory(input_dir, output_dir, model_dir, model, threshold, batch_size, mask_dir):
+@click.option('--morphology-csv', type=str, default=None,
+              help='Also measure each crop\'s instance mask (Mask R-CNN models: area, perimeter, centroid, axes, '
+                   'orientation, eccentricity, equivalent diameter, mean colour; pixels) and write one CSV row per crop')
+def infer_object_detector_directory(input_dir, output_dir, model_dir, model, threshold, batch_size, mask_dir, morphology_csv):
     model_path = os.path.join(model_dir, model, "model.pt")
     labels = read_labels(os.path.join(model_dir, model, "labels.txt"))
-    if mask_dir is None:
+    if mask_dir is None and morphology_csv is None:
         project = infer_directory_fn(input_dir, model_path, labels, threshold, batch_size)
     else:
         try:
-            project = infer_directory_fn(input_dir, model_path, labels, threshold, batch_size, with_masks=True)
+            project = infer_directory_fn(input_dir, model_path, labels, threshold, batch_size, with_masks=mask_dir is not None,
+                                         with_morphology=morphology_csv is not None)
         except ValueError as e:
             raise click.ClickException(str(e))
     Path(output_dir).mkdir(parents=True, exist_ok=True)
-    crop_objects_fn(project, output_dir, relative_to=input_dir, mask_dir=mask_dir)
+    crop_objects_fn(project, output_dir, relative_to=input_dir, mask_dir=mask_dir, morphology_csv=morphology_csv)
 
 
 if __name__ == "__main__":

@@ -24,16 +24,21 @@ def _imread(path: str) -> np.ndarray:
         return np.array(img)                       # copy: PIL-backed arrays are read-only
 
 
-def crop_objects(project: Project, output_dir: str, relative_to=None, mask_dir=None):
+def crop_objects(project: Project, output_dir: str, relative_to=None, mask_dir=None, morphology_csv=None):
     """Crops of every annotation under output_dir/<sub-folders>/<label>/. With mask_dir, each annotation's instance mask
     (`mask`, set by inference with_masks=True) is written as well, as a PNG (mode L, 0 / 255) with the crop's relative
-    path and file name under mask_dir — a separate tree, so classifiers trained on the crop folders never see it."""
+    path and file name under mask_dir — a separate tree, so classifiers trained on the crop folders never see it.
+    With morphology_csv, one CSV row per written crop, in the order the crops are written: `crop` (the crop file's path
+    relative to output_dir, with /), label, x, y, width, height, then the annotation's `morphology` (set by inference
+    with_morphology=True) in MORPHOLOGY_FIELDS order — the fields any row has; a row lacking one leaves it empty.
+    Numbers are written with repr, so they read back exactly; values are in pixels."""
     from PIL import Image
     from miso_b200 import detection
     os.makedirs(output_dir, exist_ok=True)
     output_path = Path(output_dir)
     pool = ThreadPoolExecutor(max_workers=min(16, os.cpu_count() or 1))
     pending = []
+    morph_rows = []
 
     def save(arr, target):
         Image.fromarray(arr).save(target)
@@ -81,6 +86,26 @@ def crop_objects(project: Project, output_dir: str, relative_to=None, mask_dir=N
                     mask_path = Path(mask_dir) / label_path.relative_to(output_path)
                     mask_path.mkdir(parents=True, exist_ok=True)
                     pending.append(pool.submit(save, box.mask, str(mask_path / Path(filename).with_suffix(".png"))))
+                if morphology_csv is not None:
+                    if getattr(box, "morphology", None) is None:
+                        raise ValueError(f"crop_objects: {filename} has no morphology (run inference with_morphology=True)")
+                    rel = (label_path / filename).relative_to(output_path).as_posix()
+                    morph_rows.append((rel, box.label, box.x, box.y, box.width, box.height, box.morphology))
     for f in pending:
         f.result()                      # re-raise encoder / file-system errors
     pool.shutdown()
+    if morphology_csv is not None:
+        _write_morphology_csv(morphology_csv, morph_rows)
+
+
+def _write_morphology_csv(path, rows):
+    import csv
+    from miso_b200.detection import MORPHOLOGY_FIELDS
+    fields = [f for f in MORPHOLOGY_FIELDS if any(f in r[-1] for r in rows)]
+    Path(path).parent.mkdir(parents=True, exist_ok=True)
+    with open(path, "w", newline="") as fh:
+        w = csv.writer(fh)
+        w.writerow(["crop", "label", "x", "y", "width", "height"] + fields)
+        for rel, label, x, y, width, height, m in rows:
+            w.writerow([rel, label] + [repr(float(v)) for v in (x, y, width, height)]
+                       + [repr(float(m[f])) if f in m else "" for f in fields])

@@ -7,11 +7,13 @@ import numpy as np
 
 
 class RectangleAnnotation:
-    def __init__(self, x, y, width, height, label, score=1.0, annotator=None, validator=None, uid=None, mask=None):
+    def __init__(self, x, y, width, height, label, score=1.0, annotator=None, validator=None, uid=None, mask=None,
+                 morphology=None):
         self.x, self.y, self.width, self.height = x, y, width, height
         self.label, self.score = label, score
         self.annotator, self.validator, self.uid = annotator, validator, uid
         self.mask = mask        # np.uint8 [h, w] instance mask (0 / 255) over the crop rectangle, or None
+        self.morphology = morphology    # {field: float} measurements of the mask (miso_b200.detection.MORPHOLOGY_FIELDS), or None
 
     @property
     def bounds(self):

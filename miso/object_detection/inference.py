@@ -39,15 +39,18 @@ def read_image(path) -> np.ndarray:
 
 
 def _annotate(model, images_meta: List[ImageMetadata], model_labels, threshold, batch_size, project_out: Project,
-              num_workers: int = 4, with_masks: bool = False):
+              num_workers: int = 4, with_masks: bool = False, with_morphology: bool = False):
     """One pass over the images: decode (a pool of `num_workers` threads reads and decodes the next batches while the
     GPU works — the reference uses a DataLoader with 4 workers, ref:miso/object_detection/inference.py:102-109),
     patched model, score filter + bounds on the device, annotations. with_masks (Mask R-CNN): every annotation also
     gets `mask`, its detection's instance mask over the crop rectangle (np.uint8 [h, w], 0 / 255), cut on the device
-    by the same filter_and_crop call."""
+    by the same filter_and_crop call. with_morphology (Mask R-CNN): every annotation also gets `morphology`, the
+    measurements of that mask ({field: float}, detection.MORPHOLOGY_FIELDS with the image's channel means only),
+    computed on the device as well."""
     from concurrent.futures import ThreadPoolExecutor
     from miso_b200 import detection
-    if with_masks and getattr(model.roi_heads, "mask_predictor", None) is None:
+    need_masks = with_masks or with_morphology
+    if need_masks and getattr(model.roi_heads, "mask_predictor", None) is None:
         raise ValueError("instance masks need a Mask R-CNN model; this model has no mask head")
     starts = list(range(0, len(images_meta), batch_size))
     with torch.inference_mode(), ThreadPoolExecutor(max_workers=max(1, num_workers)) as pool:
@@ -66,7 +69,7 @@ def _annotate(model, images_meta: List[ImageMetadata], model_labels, threshold, 
                 # paste per detection would be thrown away, or cut to the crop rectangles below)
                 results = forward_uint8(model, dev_u8, paste_masks=False)
             else:
-                if with_masks:
+                if need_masks:
                     raise ValueError("instance masks need a model patched by miso_b200.patch.patch_model and RGB images")
                 images_cuda = [a.permute(2, 0, 1).to(torch.float32) / 255 for a in dev_u8]       # ToTensor
                 results = model(images_cuda)
@@ -81,25 +84,30 @@ def _annotate(model, images_meta: List[ImageMetadata], model_labels, threshold, 
                     project_out.add_image(m)
                 continue
             counts = torch.tensor(counts_host, dtype=torch.int32, device="cuda")
-            probs = pad([r["mask_probs"][:, 0] for r in results], batch_first=True) if with_masks else None
+            probs = pad([r["mask_probs"][:, 0] for r in results], batch_first=True) if need_masks else None
             out = detection.filter_and_crop(dev_u8, boxes.contiguous(), scores.contiguous(), counts, threshold, capacity_bytes=0,
-                                            mask_probs=probs)
+                                            mask_probs=probs, morphology=with_morphology)
             kept = int(out.totals[0])
             masks = out.masks_to_host() if with_masks else [None] * kept
+            morph = [None] * kept
+            if with_morphology:
+                fields = detection.MORPHOLOGY_FIELDS[:len(detection.MORPHOLOGY_FIELDS) - 4 + int(dev_u8[0].shape[2])]
+                morph = [dict(zip(fields, map(float, row))) for row in out.morphology_to_host()]
             xywh = out.xywh[:kept].cpu().numpy()
             src = out.src[:kept].cpu().numpy()
             labels = labels_d.cpu().numpy()
             for j in range(kept):
                 k, d = int(src[j]) // cap, int(src[j]) % cap
                 x, y, w, h = xywh[j]
-                metas[k].boxes.append(RectangleAnnotation(x, y, w, h, model_labels[int(labels[k, d]) - 1], mask=masks[j]))
+                metas[k].boxes.append(RectangleAnnotation(x, y, w, h, model_labels[int(labels[k, d]) - 1], mask=masks[j],
+                                                           morphology=morph[j]))
             for m in metas:
                 project_out.add_image(m)
     return project_out
 
 
 def infer(project: Project, model_path: str, model_labels: List[str] = None, threshold: float = 0.5, batch_size=2,
-          nv: bool = False, with_masks: bool = False):
+          nv: bool = False, with_masks: bool = False, with_morphology: bool = False):
     if nv:
         model_labels = [label + "_NV" for label in model_labels]
     for label in model_labels:
@@ -110,11 +118,12 @@ def infer(project: Project, model_path: str, model_labels: List[str] = None, thr
     out = Project()
     for label in model_labels:
         out.add_label(None, label, None)
-    return _annotate(model, list(project.image_dict.values()), model_labels, threshold, batch_size, out, with_masks=with_masks)
+    return _annotate(model, list(project.image_dict.values()), model_labels, threshold, batch_size, out, with_masks=with_masks,
+                     with_morphology=with_morphology)
 
 
 def infer_directory(input_dir: str, model_path: str, model_labels: List[str] = None, threshold: float = 0.5, batch_size=2,
-                    with_masks: bool = False):
+                    with_masks: bool = False, with_morphology: bool = False):
     p = Path(input_dir)
     if not p.exists():
         raise ValueError(f"Directory does not exist: {input_dir}")
@@ -124,4 +133,5 @@ def infer_directory(input_dir: str, model_path: str, model_labels: List[str] = N
     out = Project()
     for label in model_labels:
         out.add_label(None, label, None)
-    return _annotate(model, metas, model_labels, threshold, batch_size, out, with_masks=with_masks)
+    return _annotate(model, metas, model_labels, threshold, batch_size, out, with_masks=with_masks,
+                     with_morphology=with_morphology)

@@ -32,6 +32,11 @@ from .ops import _f32c, _ptr, _require_cuda, _stream, _workspace, base_anchors
 BBOX_XFORM_CLIP = math.log(1000.0 / 16)
 CPU_RULE_NUMEL = 4000       # tv:ops/boxes.py:80, the reference's CPU path (the parity oracle)
 CUDA_RULE_NUMEL = 100_000   # same line, CUDA tensors
+# the columns of a crop's morphology record (mb_mask_morphology, include/misob200.h): regionprops of the crop's mask,
+# in pixels; centroids in image (or mosaic) coordinates; mean_intensity_k is 0 for k >= the image's channels
+MORPHOLOGY_FIELDS = ("area", "perimeter", "centroid_x", "centroid_y", "major_axis_length", "minor_axis_length",
+                     "orientation", "eccentricity", "equivalent_diameter",
+                     "mean_intensity_0", "mean_intensity_1", "mean_intensity_2", "mean_intensity_3")
 
 
 # ------------------------------------------------------------------------------------------
@@ -221,6 +226,7 @@ class CropOutput:
     offsets: Tensor    # [N*cap+1] int64 byte offsets into `pixels`
     pixels: Tensor     # [capacity] uint8 packed crops (HWC each)
     masks: Optional[Tensor] = None     # uint8 packed h*w masks (0 / 255) of the crops at offsets // channels
+    morphology: Optional[Tensor] = None     # [N*cap, len(MORPHOLOGY_FIELDS)] fp64 records, crop order (first totals[0] rows)
 
     def to_host(self, channels: int):
         """One device->host transfer; returns per-crop (image index, detection index, xywh, array)."""
@@ -251,6 +257,15 @@ class CropOutput:
         buf = self.masks[:tot[1] // self._ch].cpu().numpy()
         return [buf[offs[j]:offs[j + 1]].reshape(rects[j][3], rects[j][2]) for j in range(k)]
 
+    def morphology_to_host(self):
+        """The crops' morphology records as np.float64 [count, len(MORPHOLOGY_FIELDS)], crop order."""
+        if self.morphology is None:
+            raise MisoB200Error("no morphology: filter_and_crop ran without morphology=True")
+        tot = self.totals.tolist()
+        if tot[3]:
+            raise MisoB200Error(f"mask buffer too small: {tot[1] // self._ch} bytes needed")
+        return self.morphology[:tot[0]].cpu().numpy()
+
     _n: int = 1
     _ch: int = 1
 
@@ -258,14 +273,20 @@ class CropOutput:
 def filter_and_crop(images: Sequence[Tensor], det_boxes: Tensor, det_scores: Tensor, det_counts: Tensor,
                     threshold: float, capacity_bytes: Optional[int] = None, boxes_are_xywh: bool = False,
                     mask_probs: Optional[Tensor] = None, paste_boxes: Optional[Tensor] = None, mask_threshold: float = 0.5,
-                    mask_capacity_bytes: Optional[int] = None) -> CropOutput:
+                    mask_capacity_bytes: Optional[int] = None, morphology: bool = False) -> CropOutput:
     """images[n]: uint8 [H, W, C] or [H, W] on the device (the ORIGINAL image pixels, as
     skimage.io.imread returns them); det_* as produced by postprocess_detections.
 
     mask_probs ([N, cap, M, M] or [N*cap, 1, M, M], Mask R-CNN's per-detection probabilities) adds each crop's instance
     mask (mb_crop_masks): paste_masks_in_image of the detection's mask into its image at paste_boxes (default
     det_boxes, xyxy), cut to the crop rectangle, 255 where > mask_threshold else 0. capacity_bytes = 0 skips the pixel
-    gather; mask_capacity_bytes None sizes the mask buffer exactly (one host sync)."""
+    gather; mask_capacity_bytes None sizes the mask buffer exactly (one host sync).
+
+    morphology=True (needs mask_probs) also measures every crop's mask on the device (mb_mask_morphology): area,
+    perimeter, centroid, axes, orientation, eccentricity, equivalent diameter and the mean of each channel over the
+    mask, as regionprops computes them (MORPHOLOGY_FIELDS); CropOutput.morphology / morphology_to_host()."""
+    if morphology and mask_probs is None:
+        raise MisoB200Error("filter_and_crop(morphology=True) measures the instance masks: mask_probs is needed")
     lib = _lib.load()
     n, cap = det_boxes.shape[0], det_boxes.shape[1]
     if len(images) != n:
@@ -314,6 +335,12 @@ def filter_and_crop(images: Sequence[Tensor], det_boxes: Tensor, det_scores: Ten
         _lib.check(lib.mb_crop_masks(C.byref(p), _ptr(mp), _ptr(pb), m, 1, None, cap, float(mask_threshold), _ptr(rects),
                                      _ptr(src), _ptr(offsets), _ptr(totals), _ptr(masks), int(mask_capacity_bytes), st),
                    "mb_crop_masks")
-    out = CropOutput(totals, rects, xywh, src, offsets, pixels, masks)
+    morph = None
+    if morphology:
+        morph = torch.empty((n * cap, len(MORPHOLOGY_FIELDS)), dtype=torch.float64, device=dev)
+        ws = torch.empty((max(int(lib.mb_mask_morphology_workspace_bytes(C.byref(p))), 1),), dtype=torch.uint8, device=dev)
+        _lib.check(lib.mb_mask_morphology(C.byref(p), _ptr(masks), _ptr(rects), _ptr(src), _ptr(offsets), _ptr(totals),
+                                          _ptr(ws), ws.numel(), _ptr(morph), st), "mb_mask_morphology")
+    out = CropOutput(totals, rects, xywh, src, offsets, pixels, masks, morph)
     out._n, out._ch = n, ch
     return out

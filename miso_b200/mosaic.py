@@ -33,6 +33,7 @@ from torch import Tensor
 
 from . import _lib
 from ._lib import CropParams, MisoB200Error
+from .detection import MORPHOLOGY_FIELDS
 
 
 def tile_starts(extent: int, tile: int, overlap: int) -> List[int]:
@@ -216,12 +217,14 @@ class MosaicCrops:
         self.params.images[0] = band_u8.data_ptr() - self.band_y0 * band_u8.shape[1] * band_u8.shape[2]
 
     def bind_masks(self, mask_probs: Tensor, paste_boxes: Tensor, frames: Tensor, rows_per_frame: int,
-                   mask_threshold: float = 0.5) -> None:
+                   mask_threshold: float = 0.5, morphology: bool = False) -> None:
         """Cut every crop's instance mask as well (mb_crop_masks after the gather, results()["masks"]). Row s of this
         rank's block: mask_probs [rows, M, M] (maskrcnn_inference's output), paste_boxes [rows, 4] xyxy in the
         coordinates of its frame, the tile it came from: frames[s // rows_per_frame] = (x0, y0, w, h) int32 in mosaic
         coordinates. A crop's mask is the tile-sized paste_masks_in_image of its detection, cut to the crop rectangle
-        and thresholded (> mask_threshold: 255, else 0; 0 outside the tile)."""
+        and thresholded (> mask_threshold: 255, else 0; 0 outside the tile). morphology=True also measures every
+        crop's mask (mb_mask_morphology after the masks): results()["morphology"] [count, len(MORPHOLOGY_FIELDS)] fp64,
+        centroids in mosaic coordinates, channel means from the band's pixels."""
         m = int(mask_probs.shape[-1])
         for t in (mask_probs, paste_boxes, frames):
             torch._assert(t.is_cuda and t.is_contiguous(), "bind_masks: contiguous CUDA tensors expected")
@@ -232,6 +235,11 @@ class MosaicCrops:
                       and frames.shape[0] * int(rows_per_frame) >= self.rows, "bind_masks: frames must be int32 [rows / rows_per_frame, 4]")
         self.mask_args = (mask_probs, paste_boxes, frames, m, int(rows_per_frame), float(mask_threshold))
         self.masks = torch.empty((max(self.capacity // self.params.channels, 1),), dtype=torch.uint8, device=mask_probs.device)
+        self.morphology = None
+        if morphology:
+            self.morphology = torch.empty((self.rows, len(MORPHOLOGY_FIELDS)), dtype=torch.float64, device=mask_probs.device)
+            nbytes = int(self.lib.mb_mask_morphology_workspace_bytes(C.byref(self.params)))
+            self.morph_ws = torch.empty((max(nbytes, 1),), dtype=torch.uint8, device=mask_probs.device)
 
     def launch(self, gathered: Tensor, state: Tensor, row_lo: int) -> None:
         st = _cstream(gathered)
@@ -247,10 +255,15 @@ class MosaicCrops:
             _lib.check(self.lib.mb_crop_masks(cp, _p(probs), _p(boxes), m, 1, _p(frames), rpf, thr, _p(self.rects), _p(self.src),
                                               _p(self.offsets), _p(self.totals), _p(self.masks), self.masks.numel(), st),
                        "mb_crop_masks")
+            if self.morphology is not None:
+                _lib.check(self.lib.mb_mask_morphology(cp, _p(self.masks), _p(self.rects), _p(self.src), _p(self.offsets),
+                                                       _p(self.totals), _p(self.morph_ws), self.morph_ws.numel(),
+                                                       _p(self.morphology), st), "mb_mask_morphology")
 
     def results(self) -> Dict[str, Tensor]:
         """One sync: this rank's surviving detections in row order and their crop bytes; with bind_masks() also
-        "masks", the crops' h*w mask bytes packed at offsets // channels."""
+        "masks", the crops' h*w mask bytes packed at offsets // channels, and with bind_masks(morphology=True)
+        "morphology", one record per crop in the same row order."""
         tot = self.totals.tolist()
         if tot[2]:
             raise MisoB200Error(f"mosaic crop buffer too small: {tot[1]} bytes needed, {self.capacity} available")
@@ -262,6 +275,8 @@ class MosaicCrops:
                 raise MisoB200Error(f"mosaic mask buffer too small: {tot[1] // self.params.channels} bytes needed, "
                                     f"{self.masks.numel()} available")
             out["masks"] = self.masks[:tot[1] // self.params.channels]
+            if self.morphology is not None:
+                out["morphology"] = self.morphology[:k]
         return out
 
 
@@ -530,7 +545,8 @@ def by_score(gathered: Tensor, state: Tensor) -> Tensor:
 
 def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: int = 0, tile: int = 1024,
                  overlap: int = 128, threshold: float = 0.5, batch_size: int = 4, rank: int = 0, world: int = 1,
-                 group=None, crop_capacity_bytes: int = 256 << 20, masks: bool = False, mask_threshold: float = 0.5):
+                 group=None, crop_capacity_bytes: int = 256 << 20, masks: bool = False, mask_threshold: float = 0.5,
+                 morphology: bool = False):
     """Detect on a large slide/mosaic image (config 5) with a (patched) torchvision detection model: this rank runs
     its contiguous share of tiles, the per-rank detection blocks are exchanged with one all-gather, the sparse seam
     NMS runs on every rank (replicated, deterministic) and each rank cuts the crops of its own tiles' survivors.
@@ -539,10 +555,15 @@ def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: in
     rank's tiles cover (rank_band()); with world == 1 simply the whole mosaic. Returns a dict: gathered [rows, 6]
     (mosaic coordinates), state [rows] (1 = kept), and this rank's crops (MosaicCrops.results()).
     masks=True (Mask R-CNN): crops["masks"] holds every crop's instance mask, its detection's mask pasted into the
-    tile it came from, cut to the crop rectangle, > mask_threshold -> 255 (MosaicCrops.bind_masks)."""
+    tile it came from, cut to the crop rectangle, > mask_threshold -> 255 (MosaicCrops.bind_masks).
+    morphology=True (Mask R-CNN): crops["morphology"] [count, len(MORPHOLOGY_FIELDS)] fp64 on the device, each crop's
+    mask measured (area, perimeter, centroid in mosaic coordinates, axes, ...; the masks are cut for it even when
+    masks=False, and crops["masks"] is returned only when masks=True)."""
     has_mask = getattr(model.roi_heads, "mask_predictor", None) is not None
-    if masks and not has_mask:
-        raise MisoB200Error("infer_mosaic(masks=True): the model has no mask head (Mask R-CNN needed)")
+    if (masks or morphology) and not has_mask:
+        what = "masks" if masks else "morphology"
+        raise MisoB200Error(f"infer_mosaic({what}=True): the model has no mask head (Mask R-CNN needed)")
+    want_masks = masks or morphology
     dev = band_u8.device
     h, w = int(mosaic_hw[0]), int(mosaic_hw[1])
     grid = tile_grid(h, w, tile, overlap)
@@ -568,9 +589,10 @@ def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: in
                 k = int(r["boxes"].shape[0])
                 boxes[i0 + j, :k], scores[i0 + j, :k], labels[i0 + j, :k] = r["boxes"], r["scores"], r["labels"]
                 counts[i0 + j] = k
-                if masks:
+                if want_masks:
                     if "mask_probs" not in r:
-                        raise MisoB200Error("infer_mosaic(masks=True) needs a model patched by miso_b200.patch.patch_model")
+                        raise MisoB200Error("infer_mosaic(masks=True / morphology=True) needs a model patched by "
+                                            "miso_b200.patch.patch_model")
                     if probs is None:
                         m = int(r["mask_probs"].shape[-1])
                         probs = torch.zeros((tmax * dpi, m, m), dtype=torch.float32, device=dev)
@@ -587,7 +609,7 @@ def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: in
     state = seam.launch(gathered, float(model.roi_heads.nms_thresh))
     crops = MosaicCrops(tmax * dpi, (h, w), int(band_u8.shape[2]), threshold, crop_capacity_bytes, dev)
     crops.bind_band(band_u8, band_y0)
-    if masks and probs is not None:
+    if want_masks and probs is not None:
         # frame of own row s: the tile it came from (boxes are tile-local, which is what the paste wants)
         frames = torch.zeros((tmax, 4), dtype=torch.int32)
         for i, t in enumerate(mine):
@@ -595,10 +617,14 @@ def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: in
             frames[i] = torch.tensor([x, y, min(tile, w - x), min(tile, h - y)], dtype=torch.int32)
         paste_boxes = torch.zeros((tmax * dpi, 4), dtype=torch.float32, device=dev)
         paste_boxes[:len(mine) * dpi] = boxes[:len(mine)].reshape(-1, 4)
-        crops.bind_masks(probs, paste_boxes, frames.to(dev), dpi, mask_threshold)
+        crops.bind_masks(probs, paste_boxes, frames.to(dev), dpi, mask_threshold, morphology=morphology)
     crops.launch(gathered, state, rank * tmax * dpi)
     seam.check()
     res = crops.results()
-    if masks and probs is None:                    # no own tiles: no crops
+    if want_masks and probs is None:               # no own tiles: no crops
         res["masks"] = torch.empty((0,), dtype=torch.uint8, device=dev)
+        if morphology:
+            res["morphology"] = torch.empty((0, len(MORPHOLOGY_FIELDS)), dtype=torch.float64, device=dev)
+    if not masks:
+        res.pop("masks", None)
     return {"gathered": gathered, "state": state, "crops": res}
