@@ -11,7 +11,8 @@
 //   k_roi_align_nhwc4d  channels-last maps (or NCHW maps transposed once per call by k_nchw_to_nhwc
 //                       into the caller's workspace), sampling_ratio 2, <= 64 bins, C % 4 == 0:
 //                       16-byte gathers straight from global memory, taps de-duplicated per bin.
-//   k_roi_align_nhwc    channels-last, scalar gathers (14x14 mask head, odd channel counts).
+//   k_roi_align_nhwc    channels-last maps k_roi_align_nhwc4d cannot take (C % 4 != 0, maps not 16-byte
+//                       aligned, or one image's map of 4 GiB or more): scalar gathers.
 //   k_roi_align_sr2     NCHW maps without a workspace: CTA = RoI, the footprint of 32 channels is
 //                       staged NCHW -> shared memory [channel][row][col] with a plane pitch == 1
 //                       (mod 32) words so that "lane = channel" tap reads hit 32 banks.
@@ -181,19 +182,17 @@ __global__ void __launch_bounds__(kRoiThreads, 4) k_roi_align_staged(const mb_ro
                 }
             }
         }
-        if (SR2 && !direct && rows > 0) {
+        if (SR2 && !direct && rows > 0) {   // offsets of samples outside the map are never read (skipped below)
             if (tid < ph1 - ph0) {
                 const Tap a = ytab[(ph0 + tid) * 2], b = ytab[(ph0 + tid) * 2 + 1];
-                const int alo = a.valid ? a.lo : gy0, ahi = a.valid ? a.hi : gy0;
-                const int blo = b.valid ? b.lo : gy0, bhi = b.valid ? b.hi : gy0;
-                yoff2[tid] = make_int4((alo - gy0) * cols - x0, (ahi - gy0) * cols - x0,
-                                       (blo - gy0) * cols - x0, (bhi - gy0) * cols - x0);
+                yoff2[tid] = make_int4((a.lo - gy0) * cols - x0, (a.hi - gy0) * cols - x0,
+                                       (b.lo - gy0) * cols - x0, (b.hi - gy0) * cols - x0);
                 ywt2[tid] = make_float4(a.h, a.l, b.h, b.l);
             }
             if (tid >= 32 && tid < 32 + PW) {
                 const int i = tid - 32;
                 const Tap a = xtab[i * 2], b = xtab[i * 2 + 1];
-                xoff2[i] = make_int4(a.valid ? a.lo : x0, a.valid ? a.hi : x0, b.valid ? b.lo : x0, b.valid ? b.hi : x0);
+                xoff2[i] = make_int4(a.lo, a.hi, b.lo, b.hi);
                 xwt2[i] = make_float4(a.h, a.l, b.h, b.l);
             }
         }
@@ -210,11 +209,15 @@ __global__ void __launch_bounds__(kRoiThreads, 4) k_roi_align_staged(const mb_ro
                 if (c_ok && rows > 0) {
                     const int4 yo = yoff2[ph - ph0], xo = xoff2[pw];
                     const float4 yw = ywt2[ph - ph0], xw = xwt2[pw];
+                    // samples outside the map are skipped like the reference does, not weighted by 0 (an Inf / NaN
+                    // feature elsewhere cannot leak in); the branches are warp-uniform: all lanes share the bin
+                    const bool ya = ytab[2 * ph].valid, yb = ytab[2 * ph + 1].valid;
+                    const bool xa = xtab[2 * pw].valid, xb = xtab[2 * pw + 1].valid;
                     // sample (iy=0, ix=0), (0,1), (1,0), (1,1) in the reference's loop order
-                    acc = bilinear4<EXACT>(yw.x, yw.y, xw.x, xw.y, sp[yo.x + xo.x], sp[yo.x + xo.y], sp[yo.y + xo.x], sp[yo.y + xo.y], acc);
-                    acc = bilinear4<EXACT>(yw.x, yw.y, xw.z, xw.w, sp[yo.x + xo.z], sp[yo.x + xo.w], sp[yo.y + xo.z], sp[yo.y + xo.w], acc);
-                    acc = bilinear4<EXACT>(yw.z, yw.w, xw.x, xw.y, sp[yo.z + xo.x], sp[yo.z + xo.y], sp[yo.w + xo.x], sp[yo.w + xo.y], acc);
-                    acc = bilinear4<EXACT>(yw.z, yw.w, xw.z, xw.w, sp[yo.z + xo.z], sp[yo.z + xo.w], sp[yo.w + xo.z], sp[yo.w + xo.w], acc);
+                    if (ya && xa) acc = bilinear4<EXACT>(yw.x, yw.y, xw.x, xw.y, sp[yo.x + xo.x], sp[yo.x + xo.y], sp[yo.y + xo.x], sp[yo.y + xo.y], acc);
+                    if (ya && xb) acc = bilinear4<EXACT>(yw.x, yw.y, xw.z, xw.w, sp[yo.x + xo.z], sp[yo.x + xo.w], sp[yo.y + xo.z], sp[yo.y + xo.w], acc);
+                    if (yb && xa) acc = bilinear4<EXACT>(yw.z, yw.w, xw.x, xw.y, sp[yo.z + xo.x], sp[yo.z + xo.y], sp[yo.w + xo.x], sp[yo.w + xo.y], acc);
+                    if (yb && xb) acc = bilinear4<EXACT>(yw.z, yw.w, xw.z, xw.w, sp[yo.z + xo.z], sp[yo.z + xo.w], sp[yo.w + xo.z], sp[yo.w + xo.w], acc);
                 }
             } else if (c_ok && (direct || rows > 0)) {
                 for (int iy = 0; iy < g.grid_h; ++iy) {
@@ -265,12 +268,22 @@ __global__ void __launch_bounds__(kRoiThreads, 4) k_roi_align_staged(const mb_ro
 // ------------------------------------------------------------------------------------------
 constexpr int kMaxGroups = 32;
 
-template <bool EXACT>
+// A sample outside the map has negative offsets in the table (kSkipTap) and is skipped like the reference does, not
+// weighted by 0: an Inf / NaN feature elsewhere cannot leak in. Bins with all samples inside the map (nearly all) take
+// the SKIP = false body, whose loads are not split by branches; the choice is warp-uniform (lanes are channels).
+constexpr int kSkipTap = -1;
+
+__device__ __forceinline__ bool bin_all_in(const int4* __restrict__ toff) {
+    return (toff[0].x | toff[1].x | toff[2].x | toff[3].x) >= 0;
+}
+
+template <bool EXACT, bool SKIP>
 __device__ __forceinline__ float bin_value(const float* sp, const int4* __restrict__ toff, const float4* __restrict__ tw) {
     float acc = 0.0f;
 #pragma unroll
     for (int smp = 0; smp < 4; ++smp) {
         const int4 o = toff[smp];
+        if (SKIP && o.x < 0) continue;
         const float4 wv = tw[smp];
         const float v1 = sp[o.x], v2 = sp[o.y], v3 = sp[o.z], v4 = sp[o.w];
         if (EXACT) {   // ((w1*v1 + w2*v2) + w3*v3) + w4*v4, then acc + that: the reference's order
@@ -286,13 +299,14 @@ __device__ __forceinline__ float bin_value(const float* sp, const int4* __restri
     return __fmul_rn(acc, 0.25f);   // acc / 4: exact scaling
 }
 
-template <bool EXACT>
+template <bool EXACT, bool SKIP>
 __device__ __forceinline__ float bin_value_smem(unsigned sbase, const int4* __restrict__ toff, const float4* __restrict__ tw) {
     // toff holds BYTE offsets; sbase is the lane's 32-bit shared address: one add per tap
     float acc = 0.0f;
 #pragma unroll
     for (int smp = 0; smp < 4; ++smp) {
         const int4 o = toff[smp];
+        if (SKIP && o.x < 0) continue;
         const float4 wv = tw[smp];
         float v1, v2, v3, v4;
         asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v1) : "r"(sbase + o.x));
@@ -412,9 +426,10 @@ __global__ void __launch_bounds__(kRoiThreads, 4) k_roi_align_sr2(const mb_roi_a
         const bool direct = grp_direct[gi] != 0;
         const int rs = direct ? g.W : cols;                 // row stride of the addressed buffer
         const int oy = direct ? 0 : grp_y0[gi], ox = direct ? 0 : x0;
-        const int ylo = ok ? (Y.lo - oy) * rs : 0, yhi = ok ? (Y.hi - oy) * rs : 0;
-        const int xlo = ok ? X.lo - ox : 0, xhi = ok ? X.hi - ox : 0;
-        tab_off[e] = make_int4(4 * (ylo + xlo), 4 * (ylo + xhi), 4 * (yhi + xlo), 4 * (yhi + xhi));   // byte offsets
+        const int ylo = (Y.lo - oy) * rs, yhi = (Y.hi - oy) * rs;
+        const int xlo = X.lo - ox, xhi = X.hi - ox;
+        tab_off[e] = ok ? make_int4(4 * (ylo + xlo), 4 * (ylo + xhi), 4 * (yhi + xlo), 4 * (yhi + xhi))   // byte offsets
+                        : make_int4(kSkipTap, kSkipTap, kSkipTap, kSkipTap);
         tab_w[e] = ok ? make_float4(__fmul_rn(Y.h, X.h), __fmul_rn(Y.h, X.l), __fmul_rn(Y.l, X.h), __fmul_rn(Y.l, X.l))
                       : make_float4(0.f, 0.f, 0.f, 0.f);
     }
@@ -489,14 +504,17 @@ __global__ void __launch_bounds__(kRoiThreads, 4) k_roi_align_sr2(const mb_roi_a
                     for (int b = b0 + warp; b < b1; b += kRoiWarps) {
                         int4 o4[4];
                         for (int q = 0; q < 4; ++q) { o4[q] = tab_off[b * 4 + q]; o4[q].x >>= 2; o4[q].y >>= 2; o4[q].z >>= 2; o4[q].w >>= 2; }
-                        out_s[lane * opitch + b] = bin_value<EXACT>(gp, o4, tab_w + b * 4);
+                        out_s[lane * opitch + b] = bin_all_in(o4) ? bin_value<EXACT, false>(gp, o4, tab_w + b * 4)
+                                                                  : bin_value<EXACT, true>(gp, o4, tab_w + b * 4);
                     }
             } else if (P == 0) {              // no valid sample row in this group: zeros (nothing was staged)
                 for (int b = b0 + warp; b < b1; b += kRoiWarps) out_s[lane * opitch + b] = 0.0f;
             } else if (lane < nch) {
                 const unsigned sbase = smem_u32(patch + lane * pitch);    // 32-bit shared address: one add per tap
                 for (int b = b0 + warp; b < b1; b += kRoiWarps)
-                    out_s[lane * opitch + b] = bin_value_smem<EXACT>(sbase, tab_off + b * 4, tab_w + b * 4);
+                    out_s[lane * opitch + b] = bin_all_in(tab_off + b * 4)
+                                                   ? bin_value_smem<EXACT, false>(sbase, tab_off + b * 4, tab_w + b * 4)
+                                                   : bin_value_smem<EXACT, true>(sbase, tab_off + b * 4, tab_w + b * 4);
             }
             __syncthreads();
         }
@@ -524,6 +542,32 @@ __global__ void __launch_bounds__(kRoiThreads, 4) k_roi_align_sr2(const mb_roi_a
 // load/compute phases and only one barrier per chunk (output hand-over), so warps overlap their
 // own global-load latency with 16 independent loads per bin.
 // ------------------------------------------------------------------------------------------
+// one bin of k_roi_align_nhwc: toff holds BYTE offsets of the taps' pixels from the lane's channel in the image
+template <bool EXACT, bool SKIP>
+__device__ __forceinline__ float bin_value_gmem(const char* gp, const int4* __restrict__ toff, const float4* __restrict__ tw) {
+    float acc = 0.0f;
+#pragma unroll
+    for (int smp = 0; smp < 4; ++smp) {
+        const int4 o = toff[smp];
+        if (SKIP && o.x < 0) continue;
+        const float4 wv = tw[smp];
+        const float v1 = __ldg(reinterpret_cast<const float*>(gp + o.x));
+        const float v2 = __ldg(reinterpret_cast<const float*>(gp + o.y));
+        const float v3 = __ldg(reinterpret_cast<const float*>(gp + o.z));
+        const float v4 = __ldg(reinterpret_cast<const float*>(gp + o.w));
+        if (EXACT) {
+            float t = __fmul_rn(wv.x, v1);
+            t = __fadd_rn(t, __fmul_rn(wv.y, v2));
+            t = __fadd_rn(t, __fmul_rn(wv.z, v3));
+            t = __fadd_rn(t, __fmul_rn(wv.w, v4));
+            acc = __fadd_rn(acc, t);
+        } else {
+            acc = fmaf(wv.x, v1, fmaf(wv.y, v2, fmaf(wv.z, v3, fmaf(wv.w, v4, acc))));
+        }
+    }
+    return __fmul_rn(acc, 0.25f);
+}
+
 template <bool EXACT>
 __global__ void __launch_bounds__(kRoiThreads, 4) k_roi_align_nhwc(const mb_roi_align_params p,
                                                                  const float* __restrict__ rois,
@@ -561,9 +605,9 @@ __global__ void __launch_bounds__(kRoiThreads, 4) k_roi_align_nhwc(const mb_roi_
         const Tap Y = ytab[ph * 2 + (smp >> 1)], X = xtab[pw * 2 + (smp & 1)];
         const bool ok = Y.valid && X.valid;
         const int cb = C * 4;   // bytes per pixel
-        const int ylo = ok ? Y.lo * g.W : 0, yhi = ok ? Y.hi * g.W : 0;
-        const int xlo = ok ? X.lo : 0, xhi = ok ? X.hi : 0;
-        tab_off[e] = make_int4((ylo + xlo) * cb, (ylo + xhi) * cb, (yhi + xlo) * cb, (yhi + xhi) * cb);
+        const int ylo = Y.lo * g.W, yhi = Y.hi * g.W;
+        tab_off[e] = ok ? make_int4((ylo + X.lo) * cb, (ylo + X.hi) * cb, (yhi + X.lo) * cb, (yhi + X.hi) * cb)
+                        : make_int4(kSkipTap, kSkipTap, kSkipTap, kSkipTap);
         tab_w[e] = ok ? make_float4(__fmul_rn(Y.h, X.h), __fmul_rn(Y.h, X.l), __fmul_rn(Y.l, X.h), __fmul_rn(Y.l, X.l))
                       : make_float4(0.f, 0.f, 0.f, 0.f);
     }
@@ -577,26 +621,9 @@ __global__ void __launch_bounds__(kRoiThreads, 4) k_roi_align_nhwc(const mb_roi_
         if (lane < nch) {
             const char* gp = img + (size_t)(c0 + lane) * 4;
             for (int b = warp; b < nbins; b += kRoiWarps) {
-                float acc = 0.0f;
-#pragma unroll
-                for (int smp = 0; smp < 4; ++smp) {
-                    const int4 o = tab_off[b * 4 + smp];
-                    const float4 wv = tab_w[b * 4 + smp];
-                    const float v1 = __ldg(reinterpret_cast<const float*>(gp + o.x));
-                    const float v2 = __ldg(reinterpret_cast<const float*>(gp + o.y));
-                    const float v3 = __ldg(reinterpret_cast<const float*>(gp + o.z));
-                    const float v4 = __ldg(reinterpret_cast<const float*>(gp + o.w));
-                    if (EXACT) {
-                        float t = __fmul_rn(wv.x, v1);
-                        t = __fadd_rn(t, __fmul_rn(wv.y, v2));
-                        t = __fadd_rn(t, __fmul_rn(wv.z, v3));
-                        t = __fadd_rn(t, __fmul_rn(wv.w, v4));
-                        acc = __fadd_rn(acc, t);
-                    } else {
-                        acc = fmaf(wv.x, v1, fmaf(wv.y, v2, fmaf(wv.z, v3, fmaf(wv.w, v4, acc))));
-                    }
-                }
-                ob[lane * opitch + b] = __fmul_rn(acc, 0.25f);
+                const int4* to = tab_off + b * 4;
+                ob[lane * opitch + b] = bin_all_in(to) ? bin_value_gmem<EXACT, false>(gp, to, tab_w + b * 4)
+                                                       : bin_value_gmem<EXACT, true>(gp, to, tab_w + b * 4);
             }
         }
         __syncthreads();   // the chunk's bins are complete; the other buffer is free for the next chunk

@@ -644,17 +644,24 @@ k_roi_align_tma(const __grid_constant__ mb_roi_align_params p, const TmaGeom* __
 
 using namespace mb;
 
-static int g_tma_sms = 0, g_tma_smem = 0;
 static long long g_tma_launches = 0;
 extern "C" int64_t mb_roi_align_tma_launches(void) { return g_tma_launches; }
-static bool tma_device_info() {
-    if (g_tma_sms == 0) {
-        int dev = 0;
-        if (cudaGetDevice(&dev) != cudaSuccess) return false;
-        cudaDeviceGetAttribute(&g_tma_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-        cudaDeviceGetAttribute(&g_tma_sms, cudaDevAttrMultiProcessorCount, dev);
+// SM count and opt-in shared memory per block of the current device, asked once per device
+static bool tma_device_info(int& sms, int& smem) {
+    static int cached_sms[64] = {}, cached_smem[64] = {};
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return false;
+    if (cached_sms[dev] == 0) {
+        int s = 0, m = 0;
+        if (cudaDeviceGetAttribute(&m, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess ||
+            cudaDeviceGetAttribute(&s, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
+            return false;
+        cached_smem[dev] = m;
+        cached_sms[dev] = s;             // racing first calls store the same values
     }
-    return g_tma_sms > 0;
+    sms = cached_sms[dev];
+    smem = cached_smem[dev];
+    return sms > 0;
 }
 
 // static part of the envelope (no device query): what mb_roi_align_workspace_bytes can decide
@@ -674,8 +681,8 @@ size_t mb_roi_align_tma_workspace_bytes(const mb_roi_align_params& p, int64_t nu
 // records; returns 1 if launched, 0 if the caller should take the gather kernel, or an error code.
 int mb_launch_roi_align_tma(const mb_roi_align_params& p, const float* rois, int64_t num_rois, float* out,
                             int32_t* levels_out, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
-    static bool attr_set[2] = {false, false};
-    if (!p.channels_last || !tma_shape_ok(p, num_rois) || !tma_device_info()) return 0;
+    int sms = 0, smem_optin = 0;
+    if (!p.channels_last || !tma_shape_ok(p, num_rois) || !tma_device_info(sms, smem_optin)) return 0;
     if (workspace == nullptr || workspace_bytes < mb_roi_align_tma_workspace_bytes(p, num_rois)) return 0;
     if ((reinterpret_cast<uintptr_t>(out) & 15) != 0) return 0;
     for (int l = 0; l < p.num_levels; ++l) {
@@ -684,21 +691,18 @@ int mb_launch_roi_align_tma(const mb_roi_align_params& p, const float* rois, int
     }
     const unsigned ob = (unsigned)p.channels * p.pooled_h * p.pooled_w * 4u;
     const TmaSmem fixed = tma_smem_layout(0, ob);
-    if ((long long)g_tma_smem - (long long)fixed.total <= 0) return 0;
-    const unsigned ring = ((unsigned)g_tma_smem - fixed.total) / 128u * 128u;
+    if ((long long)smem_optin - (long long)fixed.total <= 0) return 0;
+    const unsigned ring = ((unsigned)smem_optin - fixed.total) / 128u * 128u;
     const unsigned row_cap = ring / 5u / 16u * 16u;        // 4 rows of one pooled row + the wrap gap always fit
     if (row_cap < 8u * (unsigned)p.channels * 4u) return 0;   // ring too small to be useful: gather kernel
     const TmaSmem L = tma_smem_layout(ring, ob);
     TmaGeom* recs = reinterpret_cast<TmaGeom*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
-    const int grid = (int)(num_rois < g_tma_sms ? num_rois : g_tma_sms);
+    const int grid = (int)(num_rois < sms ? num_rois : sms);
     const float2 ones = make_float2(1.0f, 1.0f);
     const int e = p.exact ? 1 : 0;
     static const int dbg = getenv("MB_TMA_PROBE") ? atoi(getenv("MB_TMA_PROBE")) : 0;   // development probes, see tools/roi_tma_probe.py
-    if (!attr_set[e]) {
-        MB_CUDA(e ? cudaFuncSetAttribute(k_roi_align_tma<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, g_tma_smem)
-                  : cudaFuncSetAttribute(k_roi_align_tma<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, g_tma_smem));
-        attr_set[e] = true;
-    }
+    if (e) MB_DYN_SMEM(k_roi_align_tma<true>, smem_optin);
+    else MB_DYN_SMEM(k_roi_align_tma<false>, smem_optin);
     k_roi_geom<<<(unsigned)((num_rois + 7) / 8), 256, 0, stream>>>(p, rois, (int)num_rois, row_cap, recs, levels_out, dbg);
     MB_LAUNCH_CHECK();
     if (e)

@@ -293,13 +293,9 @@ extern "C" int mb_roi_align_backward(const float* grad, const float* rois, int64
     if (!grad || !rois) return MB_ERR_INVALID_ARG;
     const long long chunks = (channels + kBwdChunk - 1) / kBwdChunk;
     if (num_rois * chunks >= (1ll << 31)) return MB_ERR_UNSUPPORTED;
-    const int patch_floats = kBwdChunk * 449;                 // footprints of up to 448 pixels per channel are staged
+    const int patch_floats = kBwdChunk * 449;                 // footprints of up to 449 pixels per channel are staged
     const int smem = patch_floats * (int)sizeof(float);
-    static bool attr = false;
-    if (!attr) {
-        MB_DYN_SMEM(k_roi_align_backward, smem);
-        attr = true;
-    }
+    MB_DYN_SMEM(k_roi_align_backward, smem);
     k_roi_align_backward<<<(unsigned)(num_rois * chunks), kBwdThreads, smem, stream>>>(
         grad, rois, spatial_scale, channels, height, width, pooled_h, pooled_w, sampling_ratio, aligned, batch_size, grad_input,
         patch_floats);
