@@ -78,6 +78,33 @@ class RpnOutput:
         return ([self.proposals[i, :c] for i, c in enumerate(cnt)], [self.scores[i, :c] for i, c in enumerate(cnt)])
 
 
+def rpn_params(cfg: RpnConfig, rpn_grids: Sequence[Tuple[int, int]], anchors_per_loc: Optional[Sequence[int]],
+               padded_image_size: Tuple[int, int], image_sizes: Sequence[Tuple[int, int]]) -> RpnParams:
+    """mb_rpn_proposals' parameters for the RPN head's output grids (H_l, W_l), without the input pointers: anchor
+    strides and base anchors (AnchorGenerator), thresholds and box-coder weights. anchors_per_loc: the head's anchors
+    per location and level, checked against the configuration when given."""
+    p = RpnParams()
+    p.num_images, p.num_levels = len(image_sizes), len(rpn_grids)
+    for l, (gh, gw) in enumerate(rpn_grids):
+        base = base_anchors(cfg.sizes[l], cfg.aspect_ratios[l])
+        a = base.shape[0]
+        if anchors_per_loc is not None:
+            torch._assert(a == anchors_per_loc[l], "anchors per location do not match the head's output channels")
+        p.feat_h[l], p.feat_w[l], p.anchors_per_loc[l] = int(gh), int(gw), a
+        p.stride_h[l], p.stride_w[l] = padded_image_size[0] // int(gh), padded_image_size[1] // int(gw)
+        for ai in range(a):
+            for c in range(4):
+                p.base_anchors[l][ai][c] = float(base[ai, c])
+    for i, (h, w) in enumerate(image_sizes):
+        p.image_h[i], p.image_w[i] = int(h), int(w)
+    p.pre_nms_top_n, p.post_nms_top_n = int(cfg.pre_nms_top_n), int(cfg.post_nms_top_n)
+    p.nms_thresh, p.score_thresh, p.min_size = float(cfg.nms_thresh), float(cfg.score_thresh), float(cfg.min_size)
+    p.wx, p.wy, p.ww, p.wh = (float(v) for v in cfg.weights)
+    p.bbox_xform_clip = float(cfg.bbox_xform_clip)
+    p.trick_numel = int(cfg.trick_numel)
+    return p
+
+
 def rpn_proposals(objectness: Sequence[Tensor], pred_bbox_deltas: Sequence[Tensor], image_sizes: Sequence[Tuple[int, int]],
                   padded_image_size: Tuple[int, int], cfg: RpnConfig, return_topk_idx: bool = False) -> RpnOutput:
     """objectness[l]: [N, A, H_l, W_l] logits, pred_bbox_deltas[l]: [N, 4A, H_l, W_l] — the RPN head's
@@ -89,32 +116,18 @@ def rpn_proposals(objectness: Sequence[Tensor], pred_bbox_deltas: Sequence[Tenso
     n = objectness[0].shape[0]
     if n > _lib.MB_MAX_IMAGES:
         raise MisoB200Error(f"rpn_proposals: at most {_lib.MB_MAX_IMAGES} images per call")
-    p = RpnParams()
-    p.num_images, p.num_levels = n, L
+    if len(image_sizes) != n:
+        raise MisoB200Error("rpn_proposals: one image size per image expected")
     keep = []
-    for l in range(L):
-        o, d = objectness[l], pred_bbox_deltas[l]
+    for o, d in zip(objectness, pred_bbox_deltas):
         _require_cuda(o, "objectness")
         _require_cuda(d, "pred_bbox_deltas")
         o, d = _f32c(o), _f32c(d)
         keep += [o, d]
-        a, gh, gw = o.shape[1], o.shape[2], o.shape[3]
-        torch._assert(d.shape == (n, 4 * a, gh, gw), "deltas must be [N, 4A, H, W]")
-        p.feat_h[l], p.feat_w[l], p.anchors_per_loc[l] = gh, gw, a
-        p.stride_h[l], p.stride_w[l] = padded_image_size[0] // gh, padded_image_size[1] // gw
-        base = base_anchors(cfg.sizes[l], cfg.aspect_ratios[l])
-        torch._assert(base.shape[0] == a, "anchors per location do not match the head's output channels")
-        for ai in range(a):
-            for c in range(4):
-                p.base_anchors[l][ai][c] = float(base[ai, c])
-        p.objectness[l], p.deltas[l] = o.data_ptr(), d.data_ptr()
-    for i, (h, w) in enumerate(image_sizes):
-        p.image_h[i], p.image_w[i] = int(h), int(w)
-    p.pre_nms_top_n, p.post_nms_top_n = int(cfg.pre_nms_top_n), int(cfg.post_nms_top_n)
-    p.nms_thresh, p.score_thresh, p.min_size = float(cfg.nms_thresh), float(cfg.score_thresh), float(cfg.min_size)
-    p.wx, p.wy, p.ww, p.wh = (float(v) for v in cfg.weights)
-    p.bbox_xform_clip = float(cfg.bbox_xform_clip)
-    p.trick_numel = int(cfg.trick_numel)
+        torch._assert(d.shape == (n, 4 * o.shape[1], o.shape[2], o.shape[3]), "deltas must be [N, 4A, H, W]")
+    p = rpn_params(cfg, [o.shape[2:] for o in keep[0::2]], [o.shape[1] for o in keep[0::2]], padded_image_size, image_sizes)
+    for l in range(L):
+        p.objectness[l], p.deltas[l] = keep[2 * l].data_ptr(), keep[2 * l + 1].data_ptr()
     dev = keep[0].device
     ws_bytes = lib.mb_rpn_workspace_bytes(C.byref(p))
     if ws_bytes == 0:
@@ -169,6 +182,23 @@ class DetOutput:
                 [self.labels[i, :c] for i, c in enumerate(cnt)])
 
 
+def det_params(cfg: DetConfig, num_images: int, num_classes: int, max_props_per_image: int,
+               image_sizes: Sequence[Tuple[int, int]], original_image_sizes: Optional[Sequence[Tuple[int, int]]] = None) -> DetParams:
+    """mb_det_postprocess' parameters. Without original_image_sizes the boxes are not rescaled to the original images."""
+    p = DetParams()
+    p.num_images, p.num_classes, p.max_props_per_image = int(num_images), int(num_classes), int(max_props_per_image)
+    p.detections_per_img = int(cfg.detections_per_img)
+    for i, (h, w) in enumerate(image_sizes):
+        p.image_h[i], p.image_w[i] = int(h), int(w)
+        if original_image_sizes is not None:
+            p.orig_h[i], p.orig_w[i] = int(original_image_sizes[i][0]), int(original_image_sizes[i][1])
+    p.nms_thresh, p.score_thresh, p.min_size = float(cfg.nms_thresh), float(cfg.score_thresh), float(cfg.min_size)
+    p.wx, p.wy, p.ww, p.wh = (float(v) for v in cfg.weights)
+    p.bbox_xform_clip = float(cfg.bbox_xform_clip)
+    p.trick_numel = int(cfg.trick_numel)
+    return p
+
+
 def postprocess_detections(class_logits: Tensor, box_regression: Tensor, proposals: Tensor, prop_counts: Tensor,
                            image_shapes: Sequence[Tuple[int, int]], cfg: DetConfig,
                            original_image_sizes: Optional[Sequence[Tuple[int, int]]] = None,
@@ -180,19 +210,8 @@ def postprocess_detections(class_logits: Tensor, box_regression: Tensor, proposa
     for t, nm in ((class_logits, "class_logits"), (box_regression, "box_regression"), (proposals, "proposals"),
                   (prop_counts, "prop_counts")):
         _require_cuda(t, nm)
-    n, r = proposals.shape[0], proposals.shape[1]
-    c = class_logits.shape[-1]
-    p = DetParams()
-    p.num_images, p.num_classes, p.max_props_per_image = n, c, r
-    p.detections_per_img = int(cfg.detections_per_img)
-    for i, (h, w) in enumerate(image_shapes):
-        p.image_h[i], p.image_w[i] = int(h), int(w)
-        if original_image_sizes is not None:
-            p.orig_h[i], p.orig_w[i] = int(original_image_sizes[i][0]), int(original_image_sizes[i][1])
-    p.nms_thresh, p.score_thresh, p.min_size = float(cfg.nms_thresh), float(cfg.score_thresh), float(cfg.min_size)
-    p.wx, p.wy, p.ww, p.wh = (float(v) for v in cfg.weights)
-    p.bbox_xform_clip = float(cfg.bbox_xform_clip)
-    p.trick_numel = int(cfg.trick_numel)
+    p = det_params(cfg, proposals.shape[0], class_logits.shape[-1], proposals.shape[1], image_shapes, original_image_sizes)
+    n = p.num_images
     ws_bytes = lib.mb_det_workspace_bytes(C.byref(p))
     if ws_bytes == 0:
         raise MisoB200Error("postprocess_detections: configuration outside the implemented envelope "
@@ -217,26 +236,122 @@ def postprocess_detections(class_logits: Tensor, box_regression: Tensor, proposa
 # ------------------------------------------------------------------------------------------
 # score filter + crops
 # ------------------------------------------------------------------------------------------
-@dataclass
-class CropOutput:
-    totals: Tensor     # [4] int64: number of crops, total bytes, pixel overflow flag, mask overflow flag
-    rects: Tensor      # [N*cap, 4] int32 (x_begin, y_begin, width, height)
-    xywh: Tensor       # [N*cap, 4] fp32 annotation bounds (x, y, w, h)
-    src: Tensor        # [N*cap] int32: n*cap + detection index
-    offsets: Tensor    # [N*cap+1] int64 byte offsets into `pixels`
-    pixels: Tensor     # [capacity] uint8 packed crops (HWC each)
-    masks: Optional[Tensor] = None     # uint8 packed h*w masks (0 / 255) of the crops at offsets // channels
-    morphology: Optional[Tensor] = None     # [N*cap, len(MORPHOLOGY_FIELDS)] fp64 records, crop order (first totals[0] rows)
+def crop_params(image_hw: Sequence[Tuple[int, int]], channels: int, capacity: int, threshold: float,
+                boxes_are_xywh: bool = False) -> CropParams:
+    """The crop kernels' parameters for images of the given (H, W), without the image pointers. capacity: detection
+    slots per image."""
+    p = CropParams()
+    p.num_images, p.capacity, p.channels = len(image_hw), int(capacity), int(channels)
+    for i, (h, w) in enumerate(image_hw):
+        p.image_h[i], p.image_w[i] = int(h), int(w)
+    p.threshold = float(threshold)
+    p.boxes_are_xywh = int(bool(boxes_are_xywh))
+    return p
+
+
+class CropStage:
+    """Score filter + crops of a batch of detections, with its parameters and fixed-capacity outputs:
+    mb_crop_plan (plan()), then mb_crop_gather, mb_crop_masks and mb_mask_morphology (cut()).
+
+    Launches neither allocate nor synchronise: every buffer is allocated by the constructor, reserve() and
+    bind_masks(), so a stage can be recorded into a CUDA graph. The bound images and mask inputs are held for as
+    long as the stage can launch. Outputs (first totals[0] rows in crop order):
+
+      totals      [4] int64: number of crops, total bytes, pixel overflow flag, mask overflow flag
+      rects       [N*cap, 4] int32 (x_begin, y_begin, width, height)
+      xywh        [N*cap, 4] fp32 annotation bounds (x, y, w, h)
+      src         [N*cap] int32: n*cap + detection index
+      offsets     [N*cap+1] int64 byte offsets into `pixels`
+      pixels      [capacity] uint8 packed crops (HWC each)
+      masks       uint8 packed h*w masks (0 / 255) of the crops at offsets // channels (bind_masks())
+      morphology  [N*cap, len(MORPHOLOGY_FIELDS)] fp64 records (bind_masks(morphology=True))
+    """
+
+    def __init__(self, image_hw: Sequence[Tuple[int, int]], channels: int, capacity: int, threshold: float, device,
+                 capacity_bytes: Optional[int] = None, boxes_are_xywh: bool = False):
+        """capacity: detection slots per image; capacity_bytes: size of the pixel buffer (None: call reserve())."""
+        self.lib = _lib.load()
+        self.params = crop_params(image_hw, channels, capacity, threshold, boxes_are_xywh)
+        self.dev = torch.device(device)
+        rows = self.params.num_images * self.params.capacity
+        self.rects = torch.zeros((rows, 4), dtype=torch.int32, device=self.dev)
+        self.xywh = torch.zeros((rows, 4), dtype=torch.float32, device=self.dev)
+        self.src = torch.zeros((rows,), dtype=torch.int32, device=self.dev)
+        self.offsets = torch.zeros((rows + 1,), dtype=torch.int64, device=self.dev)
+        self.totals = torch.zeros((4,), dtype=torch.int64, device=self.dev)
+        self.images: List[Tensor] = []
+        self.mask_args = self.masks = self.morphology = self.morph_ws = None
+        self.capacity = self.mask_capacity = 0
+        self.pixels = None
+        if capacity_bytes is not None:
+            self.reserve(capacity_bytes)
+
+    def reserve(self, capacity_bytes: int) -> None:
+        """Allocate the pixel buffer: crops that do not fit set totals[2] and are not written."""
+        self.capacity = int(capacity_bytes)
+        self.pixels = torch.empty((max(self.capacity, 1),), dtype=torch.uint8, device=self.dev)
+
+    def bind_images(self, images: Sequence[Tensor], pointers: Optional[Sequence[int]] = None) -> None:
+        """Crop from images[i] (uint8 [H, W, C] or [H, W], contiguous), addressed at pointers[i] when given (a
+        virtual base pointer of a band of rows)."""
+        self.images = list(images)
+        for i, im in enumerate(self.images):
+            self.params.images[i] = im.data_ptr() if pointers is None else int(pointers[i])
+
+    def bind_masks(self, mask_probs: Tensor, paste_boxes: Tensor, frames: Optional[Tensor], rows_per_frame: int,
+                   mask_threshold: float, capacity_bytes: int, morphology: bool = False) -> None:
+        """Cut every crop's instance mask after the pixels (mb_crop_masks): slot s pastes mask_probs[s] ([slots, M, M])
+        at paste_boxes[s] (xyxy) into frame s // rows_per_frame, frames[f] = (x0, y0, w, h) int32, or image f when
+        frames is None; > mask_threshold -> 255. morphology=True also measures every mask (mb_mask_morphology)."""
+        self.mask_args = (mask_probs, paste_boxes, frames, int(mask_probs.shape[-1]), int(rows_per_frame), float(mask_threshold))
+        self.mask_capacity = int(capacity_bytes)
+        self.masks = torch.empty((max(self.mask_capacity, 1),), dtype=torch.uint8, device=self.dev)
+        self.morphology = self.morph_ws = None
+        if morphology:
+            self.morphology = torch.empty((self.rects.shape[0], len(MORPHOLOGY_FIELDS)), dtype=torch.float64, device=self.dev)
+            nbytes = int(self.lib.mb_mask_morphology_workspace_bytes(C.byref(self.params)))
+            self.morph_ws = torch.empty((max(nbytes, 1),), dtype=torch.uint8, device=self.dev)
+
+    def plan(self, boxes: Tensor, scores: Tensor, counts: Tensor, stream) -> None:
+        """mb_crop_plan: boxes [N, cap, 4] fp32, scores [N, cap] fp32, counts [N] int32, all contiguous."""
+        _lib.check(self.lib.mb_crop_plan(C.byref(self.params), _ptr(boxes), _ptr(scores), _ptr(counts), _ptr(self.rects),
+                                         _ptr(self.xywh), _ptr(self.src), _ptr(self.offsets), _ptr(self.totals), stream),
+                   "mb_crop_plan")
+
+    def cut(self, stream) -> None:
+        """The planned crops' pixels, then (bind_masks()) their masks and morphology."""
+        cp = C.byref(self.params)
+        _lib.check(self.lib.mb_crop_gather(cp, _ptr(self.rects), _ptr(self.src), _ptr(self.offsets), _ptr(self.totals),
+                                           _ptr(self.pixels), self.capacity, stream), "mb_crop_gather")
+        if self.mask_args is None:
+            return
+        probs, boxes, frames, m, rpf, thr = self.mask_args
+        _lib.check(self.lib.mb_crop_masks(cp, _ptr(probs), _ptr(boxes), m, 1, _ptr(frames), rpf, thr, _ptr(self.rects),
+                                          _ptr(self.src), _ptr(self.offsets), _ptr(self.totals), _ptr(self.masks),
+                                          self.mask_capacity, stream), "mb_crop_masks")
+        if self.morphology is not None:
+            _lib.check(self.lib.mb_mask_morphology(cp, _ptr(self.masks), _ptr(self.rects), _ptr(self.src), _ptr(self.offsets),
+                                                   _ptr(self.totals), _ptr(self.morph_ws), self.morph_ws.numel(),
+                                                   _ptr(self.morphology), stream), "mb_mask_morphology")
+
+    def checked_totals(self, totals: Optional[Tensor] = None, pixels: bool = True, masks: bool = False) -> List[int]:
+        """totals (default: this stage's, one sync; or a host copy of them) as a list, raising if the pixel buffer
+        (pixels=True) or the mask buffer (masks=True) was too small."""
+        tot = (self.totals if totals is None else totals).tolist()
+        if pixels and tot[2]:
+            raise MisoB200Error(f"crop buffer too small: {tot[1]} bytes needed, {self.capacity} available")
+        if masks and tot[3]:
+            raise MisoB200Error(f"mask buffer too small: {tot[1] // self.params.channels} bytes needed, "
+                                f"{self.mask_capacity} available")
+        return tot
 
     def to_host(self, channels: int):
         """One device->host transfer; returns per-crop (image index, detection index, xywh, array)."""
-        tot = self.totals.tolist()
-        if tot[2]:
-            raise MisoB200Error(f"crop buffer too small: {tot[1]} bytes needed")
+        tot = self.checked_totals()
         k = tot[0]
         rects = self.rects[:k].cpu().numpy(); xywh = self.xywh[:k].cpu().numpy(); src = self.src[:k].cpu().numpy()
         offs = self.offsets[:k + 1].cpu().numpy(); pix = self.pixels[:tot[1]].cpu().numpy()
-        cap = self.rects.shape[0] // max(1, self._n)
+        cap = self.params.capacity
         out = []
         for j in range(k):
             _, _, w, h = rects[j]
@@ -248,99 +363,64 @@ class CropOutput:
         """The crops' masks as np.uint8 [h, w] arrays in crop order (one device->host transfer of the packed bytes)."""
         if self.masks is None:
             raise MisoB200Error("no masks: filter_and_crop ran without mask_probs")
-        tot = self.totals.tolist()
-        if tot[3]:
-            raise MisoB200Error(f"mask buffer too small: {tot[1] // self._ch} bytes needed")
-        k = tot[0]
+        tot = self.checked_totals(pixels=False, masks=True)
+        k, ch = tot[0], self.params.channels
         rects = self.rects[:k].cpu().numpy()
-        offs = self.offsets[:k + 1].cpu().numpy() // self._ch
-        buf = self.masks[:tot[1] // self._ch].cpu().numpy()
+        offs = self.offsets[:k + 1].cpu().numpy() // ch
+        buf = self.masks[:tot[1] // ch].cpu().numpy()
         return [buf[offs[j]:offs[j + 1]].reshape(rects[j][3], rects[j][2]) for j in range(k)]
 
     def morphology_to_host(self):
         """The crops' morphology records as np.float64 [count, len(MORPHOLOGY_FIELDS)], crop order."""
         if self.morphology is None:
             raise MisoB200Error("no morphology: filter_and_crop ran without morphology=True")
-        tot = self.totals.tolist()
-        if tot[3]:
-            raise MisoB200Error(f"mask buffer too small: {tot[1] // self._ch} bytes needed")
+        tot = self.checked_totals(pixels=False, masks=True)
         return self.morphology[:tot[0]].cpu().numpy()
-
-    _n: int = 1
-    _ch: int = 1
 
 
 def filter_and_crop(images: Sequence[Tensor], det_boxes: Tensor, det_scores: Tensor, det_counts: Tensor,
                     threshold: float, capacity_bytes: Optional[int] = None, boxes_are_xywh: bool = False,
                     mask_probs: Optional[Tensor] = None, paste_boxes: Optional[Tensor] = None, mask_threshold: float = 0.5,
-                    mask_capacity_bytes: Optional[int] = None, morphology: bool = False) -> CropOutput:
+                    mask_capacity_bytes: Optional[int] = None, morphology: bool = False) -> CropStage:
     """images[n]: uint8 [H, W, C] or [H, W] on the device (the ORIGINAL image pixels, as
     skimage.io.imread returns them); det_* as produced by postprocess_detections.
 
     mask_probs ([N, cap, M, M] or [N*cap, 1, M, M], Mask R-CNN's per-detection probabilities) adds each crop's instance
     mask (mb_crop_masks): paste_masks_in_image of the detection's mask into its image at paste_boxes (default
     det_boxes, xyxy), cut to the crop rectangle, 255 where > mask_threshold else 0. capacity_bytes = 0 skips the pixel
-    gather; mask_capacity_bytes None sizes the mask buffer exactly (one host sync).
+    gather; capacity_bytes / mask_capacity_bytes None size the buffers exactly (one host sync).
 
     morphology=True (needs mask_probs) also measures every crop's mask on the device (mb_mask_morphology): area,
     perimeter, centroid, axes, orientation, eccentricity, equivalent diameter and the mean of each channel over the
-    mask, as regionprops computes them (MORPHOLOGY_FIELDS); CropOutput.morphology / morphology_to_host()."""
+    mask, as regionprops computes them (MORPHOLOGY_FIELDS); CropStage.morphology / morphology_to_host()."""
     if morphology and mask_probs is None:
         raise MisoB200Error("filter_and_crop(morphology=True) measures the instance masks: mask_probs is needed")
-    lib = _lib.load()
     n, cap = det_boxes.shape[0], det_boxes.shape[1]
     if len(images) != n:
         raise MisoB200Error("filter_and_crop: one image per detection row expected")
-    p = CropParams()
-    p.num_images, p.capacity = n, cap
-    ch = 1 if images[0].dim() == 2 else images[0].shape[2]
-    p.channels = ch
     keep = []
-    for i, im in enumerate(images):
+    for im in images:
         _require_cuda(im, "image")
         if im.dtype != torch.uint8:
             raise MisoB200Error("filter_and_crop: images must be uint8 (HWC)")
-        im = im.contiguous()
-        keep.append(im)
-        p.image_h[i], p.image_w[i] = im.shape[0], im.shape[1]
-        p.images[i] = im.data_ptr()
-    p.threshold = float(threshold)
-    p.boxes_are_xywh = int(bool(boxes_are_xywh))
-    dev = det_boxes.device
+        keep.append(im.contiguous())
+    ch = 1 if images[0].dim() == 2 else images[0].shape[2]
+    stage = CropStage([im.shape[:2] for im in keep], ch, cap, threshold, det_boxes.device, boxes_are_xywh=boxes_are_xywh)
+    stage.bind_images(keep)
     b, s = _f32c(det_boxes), _f32c(det_scores)
-    cnt = det_counts.to(torch.int32).contiguous()
-    rects = torch.empty((n * cap, 4), dtype=torch.int32, device=dev)
-    xywh = torch.empty((n * cap, 4), dtype=torch.float32, device=dev)
-    src = torch.empty((n * cap,), dtype=torch.int32, device=dev)
-    offsets = torch.empty((n * cap + 1,), dtype=torch.int64, device=dev)
-    totals = torch.zeros((4,), dtype=torch.int64, device=dev)
     st = _stream(b)
-    _lib.check(lib.mb_crop_plan(C.byref(p), _ptr(b), _ptr(s), _ptr(cnt), _ptr(rects), _ptr(xywh), _ptr(src),
-                                _ptr(offsets), _ptr(totals), st), "mb_crop_plan")
-    if capacity_bytes is None:
-        capacity_bytes = int(totals[1].item())          # exact size: costs one host sync
-    pixels = torch.empty((max(int(capacity_bytes), 1),), dtype=torch.uint8, device=dev)
-    _lib.check(lib.mb_crop_gather(C.byref(p), _ptr(rects), _ptr(src), _ptr(offsets), _ptr(totals), _ptr(pixels),
-                                  int(capacity_bytes), st), "mb_crop_gather")
-    masks = None
+    cnt = det_counts.to(torch.int32).contiguous()
+    stage.plan(b, s, cnt, st)
+    if capacity_bytes is None or (mask_probs is not None and mask_capacity_bytes is None):
+        need = int(stage.totals[1].item())          # exact size: costs one host sync
+    stage.reserve(need if capacity_bytes is None else capacity_bytes)
     if mask_probs is not None:
         m = int(mask_probs.shape[-1])
         mp = _f32c(mask_probs)
         torch._assert(mp.numel() == n * cap * m * m and mp.shape[-2] == m, "mask_probs must be [N, cap, M, M] or [N*cap, 1, M, M]")
         pb = b if paste_boxes is None else _f32c(paste_boxes)
         torch._assert(pb.numel() == n * cap * 4, "paste_boxes must be [N, cap, 4]")
-        if mask_capacity_bytes is None:
-            mask_capacity_bytes = int(totals[1].item()) // ch
-        masks = torch.empty((max(int(mask_capacity_bytes), 1),), dtype=torch.uint8, device=dev)
-        _lib.check(lib.mb_crop_masks(C.byref(p), _ptr(mp), _ptr(pb), m, 1, None, cap, float(mask_threshold), _ptr(rects),
-                                     _ptr(src), _ptr(offsets), _ptr(totals), _ptr(masks), int(mask_capacity_bytes), st),
-                   "mb_crop_masks")
-    morph = None
-    if morphology:
-        morph = torch.empty((n * cap, len(MORPHOLOGY_FIELDS)), dtype=torch.float64, device=dev)
-        ws = torch.empty((max(int(lib.mb_mask_morphology_workspace_bytes(C.byref(p))), 1),), dtype=torch.uint8, device=dev)
-        _lib.check(lib.mb_mask_morphology(C.byref(p), _ptr(masks), _ptr(rects), _ptr(src), _ptr(offsets), _ptr(totals),
-                                          _ptr(ws), ws.numel(), _ptr(morph), st), "mb_mask_morphology")
-    out = CropOutput(totals, rects, xywh, src, offsets, pixels, masks, morph)
-    out._n, out._ch = n, ch
-    return out
+        stage.bind_masks(mp, pb, None, cap, mask_threshold, need // ch if mask_capacity_bytes is None else mask_capacity_bytes,
+                         morphology)
+    stage.cut(st)
+    return stage

@@ -32,8 +32,9 @@ import torch
 from torch import Tensor
 
 from . import _lib
-from ._lib import CropParams, MisoB200Error
-from .detection import MORPHOLOGY_FIELDS
+from ._lib import MisoB200Error
+from .detection import MORPHOLOGY_FIELDS, CropStage
+from .ops import _ptr, _stream
 
 
 def tile_starts(extent: int, tile: int, overlap: int) -> List[int]:
@@ -78,15 +79,6 @@ def gathered_row(tile_index: int, slot: int, num_tiles: int, world: int, dpi: in
     raise IndexError(tile_index)
 
 
-def _cstream(t_or_dev) -> C.c_void_p:
-    dev = t_or_dev.device if isinstance(t_or_dev, Tensor) else t_or_dev
-    return C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-
-
-def _p(t: Optional[Tensor]) -> C.c_void_p:
-    return C.c_void_p(0 if t is None else t.data_ptr())
-
-
 def pack_block(det_boxes: Tensor, det_scores: Tensor, det_labels: Tensor, det_counts: Tensor, origins: Tensor,
                threshold: float, rows: int, out: Optional[Tensor] = None) -> Tensor:
     """[T, dpi, *] detections of tiles -> [rows, 6] = (x1, y1, x2, y2, score, label) in mosaic coordinates
@@ -101,8 +93,8 @@ def pack_block(det_boxes: Tensor, det_scores: Tensor, det_labels: Tensor, det_co
         torch._assert(x.is_contiguous(), "pack_block: contiguous tensors expected")
     torch._assert(det_labels.dtype == torch.int64 and det_counts.dtype == torch.int32 and out.shape == (rows, 6),
                   "pack_block: int64 labels, int32 counts, [rows, 6] output expected")
-    _lib.check(_lib.load().mb_mosaic_pack(_p(det_boxes), _p(det_scores), _p(det_labels), _p(det_counts), _p(origins),
-                                          int(t), int(dpi), float(threshold), int(rows), _p(out), _cstream(det_boxes)),
+    _lib.check(_lib.load().mb_mosaic_pack(_ptr(det_boxes), _ptr(det_scores), _ptr(det_labels), _ptr(det_counts), _ptr(origins),
+                                          int(t), int(dpi), float(threshold), int(rows), _ptr(out), _stream(det_boxes)),
                "mb_mosaic_pack")
     return out
 
@@ -132,8 +124,8 @@ class SeamNms:
 
     def launch(self, gathered: Tensor, iou_threshold: float):
         torch._assert(gathered.is_contiguous() and gathered.shape == (self.rows, 6), "SeamNms: [rows, 6] contiguous block expected")
-        _lib.check(_lib.load().mb_mosaic_unpack(_p(gathered), self.rows, _p(self.boxes), _p(self.scores),
-                                                _p(self.labels), _cstream(gathered)), "mb_mosaic_unpack")
+        _lib.check(_lib.load().mb_mosaic_unpack(_ptr(gathered), self.rows, _ptr(self.boxes), _ptr(self.scores),
+                                                _ptr(self.labels), _stream(gathered)), "mb_mosaic_unpack")
         return self.nms(self.boxes, self.scores, self.labels, iou_threshold)
 
     def finish(self):
@@ -165,9 +157,9 @@ class SparseSeamNms:
     def launch(self, gathered: Tensor, iou_threshold: float) -> Tensor:
         torch._assert(gathered.is_contiguous() and gathered.shape == (self.rows, 6) and gathered.dtype == torch.float32,
                       "SparseSeamNms: [rows, 6] contiguous fp32 block expected")
-        _lib.check(self.lib.mb_seam_nms(_p(gathered), self.rows, self.rpt, float(iou_threshold), self.edge_cap,
-                                        _p(self.state), _p(self.keep), _p(self.status), _p(self.ws), self.ws.numel(),
-                                        _cstream(gathered)), "mb_seam_nms")
+        _lib.check(self.lib.mb_seam_nms(_ptr(gathered), self.rows, self.rpt, float(iou_threshold), self.edge_cap,
+                                        _ptr(self.state), _ptr(self.keep), _ptr(self.status), _ptr(self.ws), self.ws.numel(),
+                                        _stream(gathered)), "mb_seam_nms")
         return self.state
 
     def check(self) -> Tuple[int, int]:
@@ -178,32 +170,17 @@ class SparseSeamNms:
         return int(st[0]), int(st[1])
 
 
-class MosaicCrops:
+class MosaicCrops(CropStage):
     """One rank's share of the final stage: rows of its own block that survived the seam NMS -> annotation
     bounds, integer crop rectangles in MOSAIC coordinates, packed crop bytes cut from the rank's pixel band
-    (mb_seam_select + mb_crop_plan + mb_crop_gather; no host sync)."""
+    (mb_seam_select, then the crop stage on the mosaic as one image; no host sync)."""
 
     def __init__(self, rows: int, mosaic_hw: Tuple[int, int], channels: int, threshold: float, capacity_bytes: int, device):
-        self.lib = _lib.load()
+        super().__init__([mosaic_hw], channels, rows, threshold, device, capacity_bytes=capacity_bytes)
         self.rows = int(rows)
-        dev = device
-        self.boxes = torch.zeros((self.rows, 4), dtype=torch.float32, device=dev)
-        self.scores = torch.zeros((self.rows,), dtype=torch.float32, device=dev)
-        self.count = torch.tensor([self.rows], dtype=torch.int32, device=dev)
-        self.rects = torch.zeros((self.rows, 4), dtype=torch.int32, device=dev)
-        self.xywh = torch.zeros((self.rows, 4), dtype=torch.float32, device=dev)
-        self.src = torch.zeros((self.rows,), dtype=torch.int32, device=dev)
-        self.offsets = torch.zeros((self.rows + 1,), dtype=torch.int64, device=dev)
-        self.totals = torch.zeros((4,), dtype=torch.int64, device=dev)
-        self.capacity = int(capacity_bytes)
-        self.pixels = torch.empty((self.capacity,), dtype=torch.uint8, device=dev)
-        p = CropParams()
-        p.num_images, p.capacity, p.channels = 1, self.rows, int(channels)
-        p.image_h[0], p.image_w[0] = int(mosaic_hw[0]), int(mosaic_hw[1])
-        p.threshold = float(threshold)
-        self.params = p
-        self.band = None
-        self.mask_args = None
+        self.boxes = torch.zeros((self.rows, 4), dtype=torch.float32, device=self.dev)
+        self.scores = torch.zeros((self.rows,), dtype=torch.float32, device=self.dev)
+        self.count = torch.tensor([self.rows], dtype=torch.int32, device=self.dev)
 
     def bind_band(self, band_u8: Tensor, band_y0: int) -> None:
         """band_u8: uint8 [band_h, W, C] — mosaic rows [band_y0, band_y0 + band_h). The crop kernels address the
@@ -213,8 +190,8 @@ class MosaicCrops:
                       "bind_band: dense uint8 [h, W, C] CUDA tensor expected")
         torch._assert(band_u8.shape[1] == self.params.image_w[0] and band_u8.shape[2] == self.params.channels,
                       "bind_band: band width / channels differ from the mosaic's")
-        self.band, self.band_y0 = band_u8, int(band_y0)
-        self.params.images[0] = band_u8.data_ptr() - self.band_y0 * band_u8.shape[1] * band_u8.shape[2]
+        self.band_y0 = int(band_y0)
+        self.bind_images([band_u8], [band_u8.data_ptr() - self.band_y0 * band_u8.shape[1] * band_u8.shape[2]])
 
     def bind_masks(self, mask_probs: Tensor, paste_boxes: Tensor, frames: Tensor, rows_per_frame: int,
                    mask_threshold: float = 0.5, morphology: bool = False) -> None:
@@ -233,47 +210,25 @@ class MosaicCrops:
         torch._assert(paste_boxes.dtype == torch.float32 and paste_boxes.shape == (self.rows, 4), "bind_masks: paste_boxes must be fp32 [rows, 4]")
         torch._assert(frames.dtype == torch.int32 and frames.dim() == 2 and frames.shape[1] == 4
                       and frames.shape[0] * int(rows_per_frame) >= self.rows, "bind_masks: frames must be int32 [rows / rows_per_frame, 4]")
-        self.mask_args = (mask_probs, paste_boxes, frames, m, int(rows_per_frame), float(mask_threshold))
-        self.masks = torch.empty((max(self.capacity // self.params.channels, 1),), dtype=torch.uint8, device=mask_probs.device)
-        self.morphology = None
-        if morphology:
-            self.morphology = torch.empty((self.rows, len(MORPHOLOGY_FIELDS)), dtype=torch.float64, device=mask_probs.device)
-            nbytes = int(self.lib.mb_mask_morphology_workspace_bytes(C.byref(self.params)))
-            self.morph_ws = torch.empty((max(nbytes, 1),), dtype=torch.uint8, device=mask_probs.device)
+        super().bind_masks(mask_probs, paste_boxes, frames, rows_per_frame, mask_threshold,
+                           self.capacity // self.params.channels, morphology)
 
     def launch(self, gathered: Tensor, state: Tensor, row_lo: int) -> None:
-        st = _cstream(gathered)
-        _lib.check(self.lib.mb_seam_select(_p(gathered), _p(state), int(row_lo), self.rows, _p(self.boxes), _p(self.scores), st),
-                   "mb_seam_select")
-        cp = C.byref(self.params)
-        _lib.check(self.lib.mb_crop_plan(cp, _p(self.boxes), _p(self.scores), _p(self.count), _p(self.rects), _p(self.xywh),
-                                         _p(self.src), _p(self.offsets), _p(self.totals), st), "mb_crop_plan")
-        _lib.check(self.lib.mb_crop_gather(cp, _p(self.rects), _p(self.src), _p(self.offsets), _p(self.totals),
-                                           _p(self.pixels), self.capacity, st), "mb_crop_gather")
-        if self.mask_args is not None:
-            probs, boxes, frames, m, rpf, thr = self.mask_args
-            _lib.check(self.lib.mb_crop_masks(cp, _p(probs), _p(boxes), m, 1, _p(frames), rpf, thr, _p(self.rects), _p(self.src),
-                                              _p(self.offsets), _p(self.totals), _p(self.masks), self.masks.numel(), st),
-                       "mb_crop_masks")
-            if self.morphology is not None:
-                _lib.check(self.lib.mb_mask_morphology(cp, _p(self.masks), _p(self.rects), _p(self.src), _p(self.offsets),
-                                                       _p(self.totals), _p(self.morph_ws), self.morph_ws.numel(),
-                                                       _p(self.morphology), st), "mb_mask_morphology")
+        st = _stream(gathered)
+        _lib.check(self.lib.mb_seam_select(_ptr(gathered), _ptr(state), int(row_lo), self.rows, _ptr(self.boxes),
+                                           _ptr(self.scores), st), "mb_seam_select")
+        self.plan(self.boxes, self.scores, self.count, st)
+        self.cut(st)
 
     def results(self) -> Dict[str, Tensor]:
         """One sync: this rank's surviving detections in row order and their crop bytes; with bind_masks() also
         "masks", the crops' h*w mask bytes packed at offsets // channels, and with bind_masks(morphology=True)
         "morphology", one record per crop in the same row order."""
-        tot = self.totals.tolist()
-        if tot[2]:
-            raise MisoB200Error(f"mosaic crop buffer too small: {tot[1]} bytes needed, {self.capacity} available")
+        tot = self.checked_totals(masks=self.masks is not None)
         k = tot[0]
         out = {"count": k, "bytes": tot[1], "rects": self.rects[:k], "xywh": self.xywh[:k], "src": self.src[:k],
                "offsets": self.offsets[:k + 1], "pixels": self.pixels[:tot[1]]}
-        if self.mask_args is not None:
-            if tot[3]:
-                raise MisoB200Error(f"mosaic mask buffer too small: {tot[1] // self.params.channels} bytes needed, "
-                                    f"{self.masks.numel()} available")
+        if self.masks is not None:
             out["masks"] = self.masks[:tot[1] // self.params.channels]
             if self.morphology is not None:
                 out["morphology"] = self.morphology[:k]
@@ -335,10 +290,6 @@ class MosaicPlan:
 
     def bind_band(self, band_u8: Tensor, band_y0: int) -> None:
         self.crops.bind_band(band_u8, band_y0)
-
-    @staticmethod
-    def _c(s) -> C.c_void_p:
-        return C.c_void_p(s.cuda_stream)
 
     def capture_tiles(self, batches, serial: bool = False) -> None:
         """Record run_tiles(batches) as a CUDA graph: the ~17 launches per batch of a rank's whole tile phase then cost
@@ -408,23 +359,23 @@ class MosaicPlan:
             self.used[n][i] = True
             inp = batches(bi, n, sR) if callable(batches) else batches[bi - first if count is not None else bi]
             hp.rebind(inp["objectness"], inp["deltas"], inp["features"], inp["class_logits"], inp["box_regression"])
-            hp.rpn(self._c(sR))
+            hp.rpn(_stream(sR))
             if not serial:
                 ev["rpn"].record(sR)
                 sA.wait_event(ev["rpn"])
             if "before_roi" in hooks:
                 hooks["before_roi"](bi, hp, sA)
-            hp.roi_align(self._c(sA))
+            hp.roi_align(_stream(sA))
             if "after_roi" in hooks:
                 hooks["after_roi"](bi, hp, sA)
             if not serial:
                 ev["roi"].record(sA)
                 sD.wait_event(ev["roi"])
-            hp.detections(self._c(sD))
-            _lib.check(self.lib.mb_mosaic_pack(_p(hp.det_boxes), _p(hp.det_scores), _p(hp.det_labels), _p(hp.det_counts),
+            hp.detections(_stream(sD))
+            _lib.check(self.lib.mb_mosaic_pack(_ptr(hp.det_boxes), _ptr(hp.det_scores), _ptr(hp.det_labels), _ptr(hp.det_counts),
                                                C.c_void_p(self.origins.data_ptr() + t0 * 8), n, self.dpi, self.threshold,
                                                n * self.dpi, C.c_void_p(self.block.data_ptr() + t0 * self.dpi * 24),
-                                               self._c(sD)), "mb_mosaic_pack")
+                                               _stream(sD)), "mb_mosaic_pack")
             if not serial:
                 ev["done"].record(sD)
             if "batch_done" in hooks:
@@ -524,9 +475,7 @@ class HostMosaicRunner:
             for k, h in self.small.items():
                 h.copy_(getattr(c, k), non_blocking=True)
         self.s_out.synchronize()
-        tot = self.small["totals"].tolist()
-        if tot[2]:
-            raise MisoB200Error(f"mosaic crop buffer too small: {tot[1]} bytes needed")
+        tot = c.checked_totals(self.small["totals"])
         with torch.cuda.stream(self.s_out):
             self.pix[:tot[1]].copy_(c.pixels[:tot[1]], non_blocking=True)
         self.s_out.synchronize()

@@ -33,8 +33,11 @@ _FMT = {"xyxy": 0, "xywh": 1, "cxcywh": 2}
 # ------------------------------------------------------------------------------------------
 # plumbing
 # ------------------------------------------------------------------------------------------
-def _stream(t: Tensor) -> C.c_void_p:
-    return C.c_void_p(torch.cuda.current_stream(t.device).cuda_stream)
+def _stream(t: Union[Tensor, torch.device, torch.cuda.Stream]) -> C.c_void_p:
+    """The handle of stream `t`, or of torch's current stream on the device of tensor / device `t`."""
+    if isinstance(t, torch.cuda.Stream):
+        return C.c_void_p(t.cuda_stream)
+    return C.c_void_p(torch.cuda.current_stream(t if isinstance(t, torch.device) else t.device).cuda_stream)
 
 
 def _ptr(t: Optional[Tensor]) -> C.c_void_p:
@@ -336,6 +339,37 @@ def convert_boxes_to_roi_format(boxes: Sequence[Tensor]) -> Tensor:
     return torch.cat([ids, concat], dim=1)
 
 
+def is_channels_last(t: Tensor) -> bool:
+    """A 4-d map stored channels-last (what a torch.channels_last backbone produces), not also NCHW-contiguous."""
+    return not t.is_contiguous() and t.is_contiguous(memory_format=torch.channels_last)
+
+
+def roi_align_reads_channels_last(channels: int, output_size: Tuple[int, int], sampling_ratio: int,
+                                  dtype: torch.dtype = torch.float32) -> bool:
+    """Whether mb_multiscale_roi_align can gather from channels-last maps in place: fp32 maps with more than one
+    channel, sampling ratio 2 and pooled sides <= 16. The library rejects channels-last maps outside this envelope
+    (MB_ERR_UNSUPPORTED), so they need an NCHW copy."""
+    return (int(sampling_ratio) == 2 and int(output_size[0]) <= 16 and int(output_size[1]) <= 16 and int(channels) > 1
+            and dtype == torch.float32)
+
+
+def roi_align_params(feature_grids: Sequence[Tuple[int, int]], num_images: int, channels: int, output_size: Tuple[int, int],
+                     sampling_ratio: int, scales: Sequence[float], thresholds: Sequence[float], aligned: bool = False,
+                     exact: bool = True, channels_last: bool = False, boxes_per_image: int = 0) -> RoiAlignParams:
+    """mb_multiscale_roi_align's parameters for maps of the given (H, W) per level, without the map and count
+    pointers. scales / thresholds: pooler_levels(). boxes_per_image > 0 selects the [N, R, 4] + box_counts layout."""
+    p = RoiAlignParams()
+    p.num_levels, p.num_images, p.channels = len(feature_grids), int(num_images), int(channels)
+    p.pooled_h, p.pooled_w, p.sampling_ratio = int(output_size[0]), int(output_size[1]), int(sampling_ratio)
+    p.aligned, p.exact, p.channels_last = int(bool(aligned)), int(bool(exact)), int(bool(channels_last))
+    for l, (h, w) in enumerate(feature_grids):
+        p.height[l], p.width[l], p.spatial_scale[l] = int(h), int(w), float(scales[l])
+    for l, t in enumerate(thresholds):
+        p.level_thresholds[l] = float(t)
+    p.boxes_per_image = int(boxes_per_image)
+    return p
+
+
 def _roi_align_launch(features: Sequence[Tensor], rois: Tensor, scales: Sequence[float], thresholds: Sequence[float],
                       output_size: Tuple[int, int], sampling_ratio: int, aligned: bool, exact: bool,
                       return_levels: bool = False, use_workspace: bool = True, force_gather: bool = False,
@@ -356,28 +390,19 @@ def _roi_align_launch(features: Sequence[Tensor], rois: Tensor, scales: Sequence
     out = torch.empty((k, c, ph, pw), dtype=torch.float32, device=f0.device)
     levels = torch.empty((k,), dtype=torch.int32, device=f0.device) if return_levels else None
     if k > 0:
-        p = RoiAlignParams()
-        p.num_levels, p.num_images, p.channels = len(features), n, c
-        p.pooled_h, p.pooled_w, p.sampling_ratio = ph, pw, int(sampling_ratio)
-        p.aligned, p.exact = int(bool(aligned)), int(bool(exact))
+        nhwc = (all(f.dtype == f0.dtype and is_channels_last(f) for f in features) and
+                roi_align_reads_channels_last(c, output_size, sampling_ratio, f0.dtype))
         keepalive = []
-        # channels-last maps (what a torch.channels_last backbone produces) are consumed in place
-        nhwc = (int(sampling_ratio) == 2 and ph <= 16 and pw <= 16 and c > 1 and
-                all(f.dtype == torch.float32 and not f.is_contiguous() and
-                    f.is_contiguous(memory_format=torch.channels_last) for f in features))
-        p.channels_last = int(nhwc)
+        for f in features:
+            torch._assert(f.shape[0] == n and f.shape[1] == c, "all feature maps must share batch and channel sizes")
+            keepalive.append(f.detach() if nhwc else _f32c(f))
+        p = roi_align_params([fc.shape[2:] for fc in keepalive], n, c, output_size, sampling_ratio, scales, thresholds,
+                             aligned, exact, nhwc, per_image)
         p.force_gather = {False: 0, True: 1, 0: 0, 1: 1, 2: 2, 'auto': 0, 'gather': 1, 'tma': 2}[force_gather]
         if per_image:
-            p.boxes_per_image, p.box_counts = per_image, box_counts.data_ptr()
-        for i, f in enumerate(features):
-            torch._assert(f.shape[0] == n and f.shape[1] == c, "all feature maps must share batch and channel sizes")
-            fc = f.detach() if nhwc else _f32c(f)
-            keepalive.append(fc)
-            p.height[i], p.width[i] = fc.shape[2], fc.shape[3]
-            p.spatial_scale[i] = float(scales[i])
+            p.box_counts = box_counts.data_ptr()
+        for i, fc in enumerate(keepalive):
             p.features[i] = fc.data_ptr()
-        for i, t in enumerate(thresholds):
-            p.level_thresholds[i] = float(t)
         ws_bytes = lib.mb_roi_align_workspace_bytes(C.byref(p), k) if use_workspace else 0
         ws = _workspace(ws_bytes, f0.device) if ws_bytes else None
         rc = lib.mb_multiscale_roi_align(C.byref(p), _ptr(rois), k, _ptr(out), _ptr(levels), _ptr(ws),
@@ -433,6 +458,21 @@ def infer_scale(feature_shape: Sequence[int], original_size: Sequence[int]) -> f
     return 2 ** float(torch.tensor(approx_scale).log2().round())
 
 
+def pooler_levels(feature_grids: Sequence[Sequence[int]], image_sizes: Sequence[Tuple[int, int]],
+                  canonical_scale: int = 224, canonical_level: int = 4) -> Tuple[List[float], Tuple[float, ...]]:
+    """_setup_scales (tv:ops/poolers.py:110-134): the spatial scale of each pooler level (feature_grids: its (H, W),
+    or any shape ending in them) and the LevelMapper's area thresholds (none for a single level)."""
+    if not image_sizes:
+        raise ValueError("images list should not be empty")
+    max_x = max(s[0] for s in image_sizes)
+    max_y = max(s[1] for s in image_sizes)
+    scales = [infer_scale(g, (max_x, max_y)) for g in feature_grids]
+    k_min = int(-math.log2(scales[0]))
+    k_max = int(-math.log2(scales[-1]))
+    thresholds = level_thresholds(k_min, k_max, canonical_scale, canonical_level) if len(scales) > 1 else ()
+    return scales, thresholds
+
+
 class MultiScaleRoIAlign(torch.nn.Module):
     """Drop-in for torchvision.ops.MultiScaleRoIAlign (tv:ops/poolers.py:230-327): same
     constructor and forward(x, boxes, image_shapes); one CUDA launch for all levels."""
@@ -457,14 +497,8 @@ class MultiScaleRoIAlign(torch.nn.Module):
 
     def _setup(self, features: List[Tensor], image_shapes: List[Tuple[int, int]]) -> None:
         """_setup_scales (tv:ops/poolers.py:110-134); cached after the first call like the reference."""
-        if not image_shapes:
-            raise ValueError("images list should not be empty")
-        max_x = max(s[0] for s in image_shapes)
-        max_y = max(s[1] for s in image_shapes)
-        self.scales = [infer_scale(f.shape, (max_x, max_y)) for f in features]
-        k_min = int(-math.log2(self.scales[0]))
-        k_max = int(-math.log2(self.scales[-1]))
-        self.thresholds = level_thresholds(k_min, k_max, self.canonical_scale, self.canonical_level) if len(features) > 1 else ()
+        self.scales, self.thresholds = pooler_levels([f.shape for f in features], image_shapes, self.canonical_scale,
+                                                     self.canonical_level)
 
     def forward(self, x: Dict[str, Tensor], boxes: List[Tensor], image_shapes: List[Tuple[int, int]],
                 return_levels: bool = False):

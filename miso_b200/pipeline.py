@@ -16,7 +16,6 @@ loop around it, `HotPath.capture()` records the step as a CUDA graph.
 from __future__ import annotations
 
 import ctypes as C
-import math
 from dataclasses import dataclass
 from typing import List, Sequence, Tuple
 
@@ -24,9 +23,9 @@ import torch
 from torch import Tensor
 
 from . import _lib
-from ._lib import CropParams, DetParams, MisoB200Error, RoiAlignParams, RpnParams
-from .detection import DetConfig, RpnConfig
-from .ops import _ptr, base_anchors, infer_scale, level_thresholds
+from ._lib import MisoB200Error
+from .detection import CropStage, DetConfig, RpnConfig, det_params, rpn_params
+from .ops import _ptr, _stream, is_channels_last, pooler_levels, roi_align_params, roi_align_reads_channels_last
 
 
 @dataclass
@@ -51,6 +50,15 @@ class HotPath:
                "mb_det_postprocess": 7,       # k_det_init, k_det_candidates, k_seg_meta, k_rank_in_segment, k_nms_mask, k_nms_sweep_small, k_det_finalize
                "mb_crop_plan": 1, "mb_crop_gather": 1}
 
+    # the crop stage's outputs and capacity under the names HotPath has always had (HostPipeline's result keys)
+    crop_rects = property(lambda self: self.crop.rects)
+    crop_xywh = property(lambda self: self.crop.xywh)
+    crop_src = property(lambda self: self.crop.src)
+    crop_offsets = property(lambda self: self.crop.offsets)
+    crop_totals = property(lambda self: self.crop.totals)
+    crop_pixels = property(lambda self: self.crop.pixels)
+    crop_capacity = property(lambda self: self.crop.capacity)
+
     def __init__(self, shapes: HotPathShapes, rpn: RpnConfig, det: DetConfig, threshold: float = 0.5,
                  crop_capacity_bytes: int = 64 << 20, exact_roi_align: bool = True, device="cuda:0"):
         self.lib = _lib.load()
@@ -69,73 +77,20 @@ class HotPath:
         self.det_scores = torch.zeros((n, self.dpi), dtype=f32, device=dev)
         self.det_labels = torch.zeros((n, self.dpi), dtype=i64, device=dev)
         self.det_counts = torch.zeros((n,), dtype=i32, device=dev)
-        cap = n * self.dpi
-        self.crop_rects = torch.zeros((cap, 4), dtype=i32, device=dev)
-        self.crop_xywh = torch.zeros((cap, 4), dtype=f32, device=dev)
-        self.crop_src = torch.zeros((cap,), dtype=i32, device=dev)
-        self.crop_offsets = torch.zeros((cap + 1,), dtype=i64, device=dev)
-        self.crop_totals = torch.zeros((4,), dtype=i64, device=dev)
-        self.crop_capacity = int(crop_capacity_bytes)
-        self.crop_pixels = torch.empty((self.crop_capacity,), dtype=torch.uint8, device=dev)
+        self.crop = CropStage(shapes.original_image_sizes, shapes.image_channels, self.dpi, threshold, dev,
+                              capacity_bytes=crop_capacity_bytes)
 
-        # ---- RPN params ----
-        p = RpnParams()
-        p.num_images, p.num_levels = n, len(shapes.rpn_grids)
-        for l, (gh, gw) in enumerate(shapes.rpn_grids):
-            base = base_anchors(rpn.sizes[l], rpn.aspect_ratios[l])
-            p.feat_h[l], p.feat_w[l], p.anchors_per_loc[l] = gh, gw, base.shape[0]
-            p.stride_h[l], p.stride_w[l] = shapes.padded_image_size[0] // gh, shapes.padded_image_size[1] // gw
-            for a in range(base.shape[0]):
-                for c in range(4):
-                    p.base_anchors[l][a][c] = float(base[a, c])
-        for i, (h, w) in enumerate(shapes.image_sizes):
-            p.image_h[i], p.image_w[i] = int(h), int(w)
-        p.pre_nms_top_n, p.post_nms_top_n = int(rpn.pre_nms_top_n), R
-        p.nms_thresh, p.score_thresh, p.min_size = float(rpn.nms_thresh), float(rpn.score_thresh), float(rpn.min_size)
-        p.wx, p.wy, p.ww, p.wh = (float(v) for v in rpn.weights)
-        p.bbox_xform_clip, p.trick_numel = float(rpn.bbox_xform_clip), int(rpn.trick_numel)
-        self.rpn_params = p
-        self.anchors_per_loc = [p.anchors_per_loc[l] for l in range(p.num_levels)]
-
-        # ---- RoIAlign params ----
-        q = RoiAlignParams()
-        q.num_levels, q.num_images, q.channels = len(shapes.feature_grids), n, shapes.channels
-        q.pooled_h = q.pooled_w = shapes.pooled
-        q.sampling_ratio, q.aligned, q.exact = shapes.sampling_ratio, 0, int(exact_roi_align)
-        max_h = max(s[0] for s in shapes.image_sizes); max_w = max(s[1] for s in shapes.image_sizes)
-        scales = [infer_scale((1, 1, gh, gw), (max_h, max_w)) for gh, gw in shapes.feature_grids]
-        k_min, k_max = int(-math.log2(scales[0])), int(-math.log2(scales[-1]))
-        thr = level_thresholds(k_min, k_max) if len(scales) > 1 else ()
-        for l, (gh, gw) in enumerate(shapes.feature_grids):
-            q.height[l], q.width[l], q.spatial_scale[l] = gh, gw, scales[l]
-        for i, t in enumerate(thr):
-            q.level_thresholds[i] = t
-        q.boxes_per_image = R
-        q.box_counts = self.prop_counts.data_ptr()
-        self.roi_params = q
-
-        # ---- detection params ----
-        d = DetParams()
-        d.num_images, d.num_classes, d.max_props_per_image, d.detections_per_img = n, shapes.num_classes, R, self.dpi
-        for i in range(n):
-            d.image_h[i], d.image_w[i] = (int(v) for v in shapes.image_sizes[i])
-            d.orig_h[i], d.orig_w[i] = (int(v) for v in shapes.original_image_sizes[i])
-        d.nms_thresh, d.score_thresh, d.min_size = float(det.nms_thresh), float(det.score_thresh), float(det.min_size)
-        d.wx, d.wy, d.ww, d.wh = (float(v) for v in det.weights)
-        d.bbox_xform_clip, d.trick_numel = float(det.bbox_xform_clip), int(det.trick_numel)
-        self.det_params = d
-
-        # ---- crop params ----
-        c = CropParams()
-        c.num_images, c.capacity, c.channels = n, self.dpi, shapes.image_channels
-        for i in range(n):
-            c.image_h[i], c.image_w[i] = (int(v) for v in shapes.original_image_sizes[i])
-        c.threshold = float(threshold)
-        self.crop_params = c
+        # ---- parameter structs (the input pointers are set by bind()) ----
+        self.rpn_params = rpn_params(rpn, shapes.rpn_grids, None, shapes.padded_image_size, shapes.image_sizes)
+        scales, thresholds = pooler_levels(shapes.feature_grids, shapes.image_sizes)
+        self.roi_params = roi_align_params(shapes.feature_grids, n, shapes.channels, (shapes.pooled, shapes.pooled),
+                                           shapes.sampling_ratio, scales, thresholds, exact=exact_roi_align, boxes_per_image=R)
+        self.roi_params.box_counts = self.prop_counts.data_ptr()
+        self.det_params = det_params(det, n, shapes.num_classes, R, shapes.image_sizes, shapes.original_image_sizes)
 
         # ---- workspaces ----
-        nb = self.lib.mb_rpn_workspace_bytes(C.byref(p))
-        db = self.lib.mb_det_workspace_bytes(C.byref(d))
+        nb = self.lib.mb_rpn_workspace_bytes(C.byref(self.rpn_params))
+        db = self.lib.mb_det_workspace_bytes(C.byref(self.det_params))
         if nb == 0 or db == 0:
             raise MisoB200Error("HotPath: configuration outside the implemented envelope")
         self.rpn_ws = torch.empty((nb,), dtype=torch.uint8, device=dev)
@@ -160,7 +115,11 @@ class HotPath:
             self.rpn_params.objectness[l], self.rpn_params.deltas[l] = o.data_ptr(), dl.data_ptr()
         # FPN maps: channels-last tensors (what a torch.channels_last backbone produces) are gathered in
         # place; NCHW maps get a workspace so that the library can transpose them once per step
-        nhwc = all((not f.is_contiguous()) and f.is_contiguous(memory_format=torch.channels_last) for f in features)
+        nhwc = all(is_channels_last(f) for f in features)
+        q = self.roi_params
+        if nhwc and not roi_align_reads_channels_last(q.channels, (q.pooled_h, q.pooled_w), q.sampling_ratio, features[0].dtype):
+            raise MisoB200Error("HotPath.bind: mb_multiscale_roi_align cannot read these channels-last maps in place "
+                                "(fp32, channels > 1, sampling ratio 2, pooled sides <= 16); bind NCHW maps")
         self.roi_params.channels_last = int(nhwc)
         for l, f in enumerate(features):
             self.roi_params.features[l] = f.data_ptr()
@@ -168,8 +127,7 @@ class HotPath:
         self.roi_ws = torch.empty((nb,), dtype=torch.uint8, device=self.dev) if nb else None
         self.features_layout = "channels_last" if nhwc else "nchw"
         self.kernel_launches_per_step = sum(self.KERNELS.values()) + (len(features) if (nb and not nhwc) else 0)   # + k_nchw_to_nhwc per level
-        for i, im in enumerate(images):
-            self.crop_params.images[i] = im.data_ptr()
+        self.crop.bind_images(images)
         self.class_logits, self.box_regression = class_logits, box_regression
         self._graph = None                               # a captured graph refers to the previous tensors
 
@@ -191,24 +149,21 @@ class HotPath:
         self.box_regression = box_regression[0] if isinstance(box_regression, (list, tuple)) else box_regression
         self._graph = None
 
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.dev).cuda_stream)
-
     def rpn(self, st=None):
-        st = st or self._stream()
+        st = st or _stream(self.dev)
         _lib.check(self.lib.mb_rpn_proposals(C.byref(self.rpn_params), _ptr(self.proposals), _ptr(self.prop_scores),
                                              _ptr(self.prop_counts), None, _ptr(self.rpn_ws), self.rpn_ws.numel(), st),
                    "mb_rpn_proposals")
 
     def roi_align(self, st=None):
-        st = st or self._stream()
+        st = st or _stream(self.dev)
         _lib.check(self.lib.mb_multiscale_roi_align(C.byref(self.roi_params), _ptr(self.proposals),
                                                     self.s.num_images * self.R, _ptr(self.box_features), None,
                                                     _ptr(self.roi_ws), self.roi_ws.numel() if self.roi_ws is not None else 0, st),
                    "mb_multiscale_roi_align")
 
     def detections(self, st=None):
-        st = st or self._stream()
+        st = st or _stream(self.dev)
         _lib.check(self.lib.mb_det_postprocess(C.byref(self.det_params), _ptr(self.class_logits), _ptr(self.box_regression),
                                                _ptr(self.proposals), _ptr(self.prop_counts), 0, _ptr(self.det_boxes),
                                                _ptr(self.det_boxes_net), _ptr(self.det_scores), _ptr(self.det_labels),
@@ -216,17 +171,12 @@ class HotPath:
                    "mb_det_postprocess")
 
     def crops(self, st=None):
-        st = st or self._stream()
-        cp = C.byref(self.crop_params)
-        _lib.check(self.lib.mb_crop_plan(cp, _ptr(self.det_boxes), _ptr(self.det_scores), _ptr(self.det_counts),
-                                         _ptr(self.crop_rects), _ptr(self.crop_xywh), _ptr(self.crop_src),
-                                         _ptr(self.crop_offsets), _ptr(self.crop_totals), st), "mb_crop_plan")
-        _lib.check(self.lib.mb_crop_gather(cp, _ptr(self.crop_rects), _ptr(self.crop_src), _ptr(self.crop_offsets),
-                                           _ptr(self.crop_totals), _ptr(self.crop_pixels), self.crop_capacity, st),
-                   "mb_crop_gather")
+        st = st or _stream(self.dev)
+        self.crop.plan(self.det_boxes, self.det_scores, self.det_counts, st)
+        self.crop.cut(st)
 
     def step(self) -> None:
-        st = self._stream()
+        st = _stream(self.dev)
         self.rpn(st)
         self.roi_align(st)
         self.detections(st)
@@ -256,21 +206,11 @@ class HotPath:
     def results(self):
         """Read back one step's results (one sync): per-image detections that passed the score
         filter, their annotation bounds and crop arrays."""
-        tot = self.crop_totals.tolist()
-        if tot[2]:
-            raise MisoB200Error(f"crop buffer too small: {tot[1]} bytes needed, {self.crop_capacity} available")
-        k = tot[0]
-        rects = self.crop_rects[:k].cpu().numpy(); xywh = self.crop_xywh[:k].cpu().numpy()
-        src = self.crop_src[:k].cpu().numpy(); offs = self.crop_offsets[:k + 1].cpu().numpy()
-        pix = self.crop_pixels[:tot[1]].cpu().numpy()
-        labels = self.det_labels.cpu().numpy().reshape(-1); scores = self.det_scores.cpu().numpy().reshape(-1)
-        ch = self.s.image_channels
+        crops = self.crop.to_host(self.s.image_channels)
+        labels = self.det_labels.cpu().numpy(); scores = self.det_scores.cpu().numpy()
         out = [[] for _ in range(self.s.num_images)]
-        for j in range(k):
-            _, _, w, h = rects[j]
-            arr = pix[offs[j]:offs[j + 1]].reshape((h, w, ch) if ch > 1 else (h, w))
-            out[int(src[j]) // self.dpi].append({"xywh": xywh[j], "label": int(labels[src[j]]),
-                                                "score": float(scores[src[j]]), "crop": arr})
+        for i, d, xywh, arr in crops:
+            out[i].append({"xywh": xywh, "label": int(labels[i, d]), "score": float(scores[i, d]), "crop": arr})
         return out
 
 
@@ -319,10 +259,7 @@ class HostPipeline:
         if slot["state"] != "small":
             return
         slot["ev"]["small"].synchronize()
-        tot = slot["out"]["crop_totals"]
-        if int(tot[2]):
-            raise MisoB200Error(f"crop buffer too small: {int(tot[1])} bytes needed")
-        nb = slot["nb"] = int(tot[1])
+        nb = slot["nb"] = slot["hp"].crop.checked_totals(slot["out"]["crop_totals"])[1]
         with torch.cuda.stream(self.s_out):
             slot["pix"][:nb].copy_(slot["hp"].crop_pixels[:nb], non_blocking=True)
             slot["ev"]["pix"].record(self.s_out)
@@ -404,9 +341,6 @@ class OverlappedHotPath:
         self.hooks = {}          # "before_roi" / "after_roi" / "before_det" / "after_det": fn(slot_index, hp, stream) —
                                  # timing events, the mosaic exchange; hooks that enqueue work must use `stream` explicitly
 
-    def _c(self, s):
-        return C.c_void_p(s.cuda_stream)
-
     def submit(self) -> int:
         i = self.k % len(self.hps)
         hp, ev = self.hps[i], self.ev[i]
@@ -419,22 +353,22 @@ class OverlappedHotPath:
         self.used[i] = True
         hooks = self.hooks
         # explicit stream handles everywhere (no stream context switches on the host)
-        hp.rpn(self._c(self.sR))
+        hp.rpn(_stream(self.sR))
         ev["rpn"].record(self.sR)
         self.sA.wait_event(ev["rpn"])
         if "before_roi" in hooks:
             hooks["before_roi"](i, hp, self.sA)
-        hp.roi_align(self._c(self.sA))
+        hp.roi_align(_stream(self.sA))
         ev["roi"].record(self.sA)
         if "after_roi" in hooks:
             hooks["after_roi"](i, hp, self.sA)
         self.sD.wait_event(ev["roi"])
         if "before_det" in hooks:
             hooks["before_det"](i, hp, self.sD)
-        hp.detections(self._c(self.sD))
+        hp.detections(_stream(self.sD))
         if "after_det" in hooks:
             hooks["after_det"](i, hp, self.sD)
-        hp.crops(self._c(self.sD))
+        hp.crops(_stream(self.sD))
         ev["done"].record(self.sD)
         self.k += 1
         return i

@@ -96,6 +96,25 @@ def check_against_oracle(w, hp):
         assert len(res[i]) == len(ref[i]["crops"])
 
 
+def test_hot_path_bind_rejects_channels_last_maps_outside_the_in_place_envelope():
+    """Channels-last FPN maps that mb_multiscale_roi_align cannot read in place (here: sampling ratio 0) are refused by
+    bind(); HotPath allocates nothing per step, so it cannot fall back to an NCHW copy."""
+    import dataclasses
+    from miso_b200 import pipeline, workload
+    from miso_b200._lib import MisoB200Error
+    w = workload.faster_rcnn_batch(num_images=1, original=320, resized=256, channels=16, post_nms_top_n=200,
+                                   detections_per_img=50, pin=False, features_layout="channels_last")
+    hp = pipeline.HotPath(dataclasses.replace(w.shapes, sampling_ratio=0), w.rpn, w.det, crop_capacity_bytes=1 << 20, device=DEV)
+    d = workload.to_device(w, DEV)
+    with pytest.raises(MisoB200Error, match="channels-last"):
+        hp.bind(d["objectness"], d["deltas"], d["features"], d["class_logits"][0], d["box_regression"][0], d["images"])
+    nchw = [f.contiguous() for f in d["features"]]
+    hp.bind(d["objectness"], d["deltas"], nchw, d["class_logits"][0], d["box_regression"][0], d["images"])
+    hp.step()
+    torch.cuda.synchronize()
+    assert hp.features_layout == "nchw"
+
+
 def test_hot_path_is_deterministic_and_idempotent():
     w, hp = build(seed=3)
     hp.step(); torch.cuda.synchronize()

@@ -23,7 +23,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from miso_b200 import _lib, mosaic  # noqa: E402
-from miso_b200.mosaic import _cstream, _p  # noqa: E402
+from miso_b200.ops import _ptr, _stream  # noqa: E402
 from tests import cases  # noqa: E402
 
 DEV = "cuda:0"
@@ -67,11 +67,11 @@ def main(reps: int = 50) -> None:
     k, mask_bytes = res["count"], res["bytes"] // 3
     assert k == rows, (k, rows)
 
-    lib, st = crops.lib, _cstream(gathered)
+    lib, st = crops.lib, _stream(gathered)
 
     def launch():
-        _lib.check(lib.mb_crop_masks(C.byref(crops.params), _p(probs), _p(boxes), M, 1, _p(frames), DPI, 0.5, _p(crops.rects),
-                                     _p(crops.src), _p(crops.offsets), _p(crops.totals), _p(crops.masks),
+        _lib.check(lib.mb_crop_masks(C.byref(crops.params), _ptr(probs), _ptr(boxes), M, 1, _ptr(frames), DPI, 0.5, _ptr(crops.rects),
+                                     _ptr(crops.src), _ptr(crops.offsets), _ptr(crops.totals), _ptr(crops.masks),
                                      crops.masks.numel(), st), "mb_crop_masks")
     for _ in range(5):
         launch()

@@ -23,7 +23,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from miso_b200 import _lib, mosaic  # noqa: E402
-from miso_b200.mosaic import _cstream, _p  # noqa: E402
+from miso_b200.ops import _ptr, _stream  # noqa: E402
 from tests import cases  # noqa: E402
 
 DEV = "cuda:0"
@@ -69,12 +69,12 @@ def main(reps: int = 50) -> None:
     area = res["morphology"][:, 0].clone()
     lit = float(area.sum()) / mask_bytes
 
-    lib, st = crops.lib, _cstream(gathered)
+    lib, st = crops.lib, _stream(gathered)
 
     def launch():
-        _lib.check(lib.mb_mask_morphology(C.byref(crops.params), _p(crops.masks), _p(crops.rects), _p(crops.src),
-                                          _p(crops.offsets), _p(crops.totals), _p(crops.morph_ws), crops.morph_ws.numel(),
-                                          _p(crops.morphology), st), "mb_mask_morphology")
+        _lib.check(lib.mb_mask_morphology(C.byref(crops.params), _ptr(crops.masks), _ptr(crops.rects), _ptr(crops.src),
+                                          _ptr(crops.offsets), _ptr(crops.totals), _ptr(crops.morph_ws), crops.morph_ws.numel(),
+                                          _ptr(crops.morphology), st), "mb_mask_morphology")
     for _ in range(5):
         launch()
     torch.cuda.synchronize()
