@@ -335,6 +335,38 @@ size_t mb_mask_morphology_workspace_bytes(const mb_crop_params* params_host);
 int mb_mask_morphology(const mb_crop_params* params_host, const uint8_t* masks, const int32_t* rects,
                        const int32_t* src, const int64_t* offsets, const int64_t* totals, void* workspace,
                        size_t workspace_bytes, double* out, mb_stream_t stream);
+/* Lossless PNG files of the packed crops (mb_crop_gather, channels == params.channels) or masks (mb_crop_masks,
+ * channels == 1): one complete stream per crop, packed in crop order at png_offsets_out[j]
+ * ([num_images*capacity + 1] int64; crop j is png_offsets_out[j + 1] - png_offsets_out[j] bytes, 0 when h*w == 0).
+ * Crop j (rect (x, y, w, h)) is read at packed + offsets[j] / params.channels * channels, h*w*channels bytes.
+ * The bytes depend only on the crop's pixels, h, w and channels:
+ *   framing  PNG signature, IHDR (w, h, bit depth 8, colour type 0 / 4 / 2 / 6 for 1 / 2 / 3 / 4 channels, no
+ *            interlace), one IDAT, IEND; no other chunks
+ *   filter   per row, the type 0..4 with the least sum over the row of |(int8) filtered byte| (ties: lower type);
+ *            row -1 is zeros
+ *   zlib     header 78 01; the filtered bytes (h * (1 + w*channels)) cut every 32768 bytes into blocks coded
+ *            independently; each block is non-final and followed by an empty stored block; the stream ends with an
+ *            empty final fixed-Huffman block (03 00) and the Adler-32 of the filtered bytes
+ *   tokens   per maximal run of n equal bytes inside a block: a literal, then the n - 1 repeats as length-258
+ *            matches at distance 1, then the m = (n - 1) % 258 left: one match of length m if m >= 3, else m literals
+ *   codes    dynamic per block: lengths by package-merge (limit 15; 7 for the code-length code) over the used symbols
+ *            sorted by (frequency, index), leaves before packages of equal weight; fewer than two used symbols: the
+ *            lowest unused indices get length 1 too (the distance code is always [1, 1]); HLIT = last used literal /
+ *            length symbol + 1, HDIST = 2; the code lengths run-length coded per tree by zlib's scan_tree / send_tree
+ *   stored   a block whose dynamic form plus its empty stored block is not shorter than L + 10 bytes (the block
+ *            stored, plus the empty stored block) is stored
+ * mb_png_bound_bytes: a capacity no packed set of `crops` crops of packed_bytes bytes (h*w*channels summed) can
+ *   exceed: 75 * crops + F + 10 * (F / 32768) with F = packed_bytes + ceil(packed_bytes / channels); -1 for bad input.
+ * mb_png_workspace_bytes: for packed crops of up to packed_capacity_bytes (h*w*channels summed); 0 for bad input.
+ * png_status_out [2] int64: [0] total bytes, [1] 1 if that exceeds png_capacity_bytes (nothing is written), 2 if the
+ * workspace is too small for the crops (nothing is encoded), else 0. A pixel or mask overflow flag in totals (totals[2],
+ * totals[3]) means nothing is encoded (no crops). Channels outside 1..4: MB_ERR_UNSUPPORTED. */
+int64_t mb_png_bound_bytes(int64_t packed_bytes, int64_t crops, int32_t channels);
+size_t mb_png_workspace_bytes(const mb_crop_params* params_host, int64_t packed_capacity_bytes, int32_t channels);
+int mb_png_encode(const mb_crop_params* params_host, const uint8_t* packed, int32_t channels, const int32_t* rects,
+                  const int64_t* offsets, const int64_t* totals, void* workspace, size_t workspace_bytes,
+                  uint8_t* png_out, int64_t png_capacity_bytes, int64_t* png_offsets_out, int64_t* png_status_out,
+                  mb_stream_t stream);
 /* maskrcnn_inference (tv:models/detection/roi_heads.py:56-82): mask_logits [R, C, M, M], labels [R] int64 ->
  * out [R, 1, M, M] = sigmoid(mask_logits[r, labels[r]]). Labels outside [0, C) are the caller's error. */
 int mb_mask_prob(const float* mask_logits, const int64_t* labels, int64_t num_masks, int32_t num_classes,

@@ -24,14 +24,18 @@ def _imread(path: str) -> np.ndarray:
         return np.array(img)                       # copy: PIL-backed arrays are read-only
 
 
-def crop_objects(project: Project, output_dir: str, relative_to=None, mask_dir=None, morphology_csv=None):
+def crop_objects(project: Project, output_dir: str, relative_to=None, mask_dir=None, morphology_csv=None,
+                 png_on_gpu=False):
     """Crops of every annotation under output_dir/<sub-folders>/<label>/. With mask_dir, each annotation's instance mask
     (`mask`, set by inference with_masks=True) is written as well, as a PNG (mode L, 0 / 255) with the crop's relative
     path and file name under mask_dir — a separate tree, so classifiers trained on the crop folders never see it.
     With morphology_csv, one CSV row per written crop, in the order the crops are written: `crop` (the crop file's path
     relative to output_dir, with /), label, x, y, width, height, then the annotation's `morphology` (set by inference
     with_morphology=True) in MORPHOLOGY_FIELDS order — the fields any row has; a row lacking one leaves it empty.
-    Numbers are written with repr, so they read back exactly; values are in pixels."""
+    Numbers are written with repr, so they read back exactly; values are in pixels.
+    png_on_gpu=True encodes the crops of .png sources (any case) that are uint8 with 1..4 channels on the device
+    (mb_png_encode, lossless: the same pixels as PIL's files, other bytes); the pool then only writes the files. Other
+    sources and the mask files keep PIL."""
     from PIL import Image
     from miso_b200 import detection
     os.makedirs(output_dir, exist_ok=True)
@@ -42,6 +46,10 @@ def crop_objects(project: Project, output_dir: str, relative_to=None, mask_dir=N
 
     def save(arr, target):
         Image.fromarray(arr).save(target)
+
+    def write(data, target):
+        with open(target, "wb") as fh:
+            fh.write(data)
 
     for image in project.image_dict.values():
         if len(image.boxes) == 0:
@@ -63,11 +71,14 @@ def crop_objects(project: Project, output_dir: str, relative_to=None, mask_dir=N
         bounds = torch.tensor(corners, dtype=torch.float32, device="cuda")
         scores = torch.ones((1, k), dtype=torch.float32, device="cuda")
         counts = torch.tensor([k], dtype=torch.int32, device="cuda")
-        out = detection.filter_and_crop([dev], bounds[None], scores, counts, 0.5, boxes_are_xywh=False)
+        path = Path(image.full_path)
+        on_gpu = png_on_gpu and path.suffix.lower() == ".png" and im.dtype == np.uint8 and 1 <= bpp <= 4
+        out = detection.filter_and_crop([dev], bounds[None], scores, counts, 0.5, boxes_are_xywh=False,
+                                        **({"png": True} if on_gpu else {}))
+        encoded = out.png_to_host() if on_gpu else None
         crops = [(n, i, xywh, np.ascontiguousarray(c).reshape(c.shape[0], c.shape[1], bpp).view(im.dtype).reshape(c.shape[:2] + px_shape))
                  for n, i, xywh, c in out.to_host(bpp)]
-        path = Path(image.full_path)
-        for (_, idx, _xywh, crop), box in zip(crops, image.boxes):
+        for j, ((_, idx, _xywh, crop), box) in enumerate(zip(crops, image.boxes)):
             if relative_to is not None:
                 label_path = output_path / path.relative_to(relative_to).parent / box.label
             elif len(project.task_names) > 0:
@@ -78,7 +89,8 @@ def crop_objects(project: Project, output_dir: str, relative_to=None, mask_dir=N
             s = box.bounds
             filename = f"{path.stem}_{s[0]:.0f}_{s[1]:.0f}_{s[2]:.0f}_{s[3]:.0f}{path.suffix}"
             if crop.size:
-                pending.append(pool.submit(save, crop, os.path.join(str(label_path), filename)))
+                target = os.path.join(str(label_path), filename)
+                pending.append(pool.submit(write, encoded[j], target) if on_gpu else pool.submit(save, crop, target))
                 if mask_dir is not None and getattr(box, "mask", None) is not None:
                     if box.mask.shape != crop.shape[:2]:
                         raise ValueError(f"crop_objects: mask {box.mask.shape} of {filename} differs from its crop "

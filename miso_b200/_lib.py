@@ -116,6 +116,9 @@ SIGNATURES = {
     "mb_crop_masks": (C.c_int, [C.POINTER(CropParams), _p, _p, _i32, _i32, _p, _i32, _f32, _p, _p, _p, _p, _p, _i64, _p]),
     "mb_mask_morphology_workspace_bytes": (_sz, [C.POINTER(CropParams)]),
     "mb_mask_morphology": (C.c_int, [C.POINTER(CropParams), _p, _p, _p, _p, _p, _p, _sz, _p, _p]),
+    "mb_png_bound_bytes": (_i64, [_i64, _i64, _i32]),
+    "mb_png_workspace_bytes": (_sz, [C.POINTER(CropParams), _i64, _i32]),
+    "mb_png_encode": (C.c_int, [C.POINTER(CropParams), _p, _i32, _p, _p, _p, _p, _sz, _p, _i64, _p, _p, _p]),
     "mb_image_transform": (C.c_int, [C.POINTER(TransformParams), _p, _p]),
 }
 

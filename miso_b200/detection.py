@@ -265,6 +265,8 @@ class CropStage:
       pixels      [capacity] uint8 packed crops (HWC each)
       masks       uint8 packed h*w masks (0 / 255) of the crops at offsets // channels (bind_masks())
       morphology  [N*cap, len(MORPHOLOGY_FIELDS)] fp64 records (bind_masks(morphology=True))
+      png, png_offsets, png_status          one PNG file per crop, packed in crop order (bind_png(), mb_png_encode);
+      mask_png, mask_png_offsets, mask_png_status   the same for the masks (bind_png() with bind_masks())
     """
 
     def __init__(self, image_hw: Sequence[Tuple[int, int]], channels: int, capacity: int, threshold: float, device,
@@ -283,6 +285,7 @@ class CropStage:
         self.mask_args = self.masks = self.morphology = self.morph_ws = None
         self.capacity = self.mask_capacity = 0
         self.pixels = None
+        self.png = self.mask_png = None
         if capacity_bytes is not None:
             self.reserve(capacity_bytes)
 
@@ -307,10 +310,39 @@ class CropStage:
         self.mask_capacity = int(capacity_bytes)
         self.masks = torch.empty((max(self.mask_capacity, 1),), dtype=torch.uint8, device=self.dev)
         self.morphology = self.morph_ws = None
+        if self.png is not None:
+            self.mask_png = self._png_buffers(self.mask_capacity, 1, self._mask_png_capacity)
         if morphology:
             self.morphology = torch.empty((self.rects.shape[0], len(MORPHOLOGY_FIELDS)), dtype=torch.float64, device=self.dev)
             nbytes = int(self.lib.mb_mask_morphology_workspace_bytes(C.byref(self.params)))
             self.morph_ws = torch.empty((max(nbytes, 1),), dtype=torch.uint8, device=self.dev)
+
+    def bind_png(self, capacity_bytes: Optional[int] = None, mask_capacity_bytes: Optional[int] = None) -> None:
+        """Encode every crop as a PNG file after the cut (mb_png_encode), and every mask when bind_masks() is (or gets)
+        called. Capacities default to mb_png_bound_bytes of the pixel / mask buffers, which no crop set can exceed."""
+        self.png = self._png_buffers(self.capacity, self.params.channels, capacity_bytes)
+        self._mask_png_capacity = mask_capacity_bytes
+        if self.masks is not None:
+            self.mask_png = self._png_buffers(self.mask_capacity, 1, mask_capacity_bytes)
+
+    def _png_buffers(self, packed_capacity: int, channels: int, capacity_bytes: Optional[int]) -> dict:
+        slots = self.rects.shape[0]
+        if capacity_bytes is None:
+            capacity_bytes = int(self.lib.mb_png_bound_bytes(packed_capacity, slots, channels))
+        ws = int(self.lib.mb_png_workspace_bytes(C.byref(self.params), packed_capacity, channels))
+        if capacity_bytes < 0 or ws == 0:
+            raise MisoB200Error(f"mb_png_encode: {channels} channels are not supported (1..4)")
+        return {"channels": channels, "capacity": int(capacity_bytes),
+                "out": torch.empty((max(int(capacity_bytes), 1),), dtype=torch.uint8, device=self.dev),
+                "offsets": torch.zeros((slots + 1,), dtype=torch.int64, device=self.dev),
+                "status": torch.zeros((2,), dtype=torch.int64, device=self.dev),
+                "ws": torch.empty((ws,), dtype=torch.uint8, device=self.dev)}
+
+    def _encode(self, buf: dict, packed: Tensor, stream) -> None:
+        _lib.check(self.lib.mb_png_encode(C.byref(self.params), _ptr(packed), buf["channels"], _ptr(self.rects),
+                                          _ptr(self.offsets), _ptr(self.totals), _ptr(buf["ws"]), buf["ws"].numel(),
+                                          _ptr(buf["out"]), buf["capacity"], _ptr(buf["offsets"]), _ptr(buf["status"]),
+                                          stream), "mb_png_encode")
 
     def plan(self, boxes: Tensor, scores: Tensor, counts: Tensor, stream) -> None:
         """mb_crop_plan: boxes [N, cap, 4] fp32, scores [N, cap] fp32, counts [N] int32, all contiguous."""
@@ -324,6 +356,8 @@ class CropStage:
         _lib.check(self.lib.mb_crop_gather(cp, _ptr(self.rects), _ptr(self.src), _ptr(self.offsets), _ptr(self.totals),
                                            _ptr(self.pixels), self.capacity, stream), "mb_crop_gather")
         if self.mask_args is None:
+            if self.png is not None:
+                self._encode(self.png, self.pixels, stream)
             return
         probs, boxes, frames, m, rpf, thr = self.mask_args
         _lib.check(self.lib.mb_crop_masks(cp, _ptr(probs), _ptr(boxes), m, 1, _ptr(frames), rpf, thr, _ptr(self.rects),
@@ -333,6 +367,11 @@ class CropStage:
             _lib.check(self.lib.mb_mask_morphology(cp, _ptr(self.masks), _ptr(self.rects), _ptr(self.src), _ptr(self.offsets),
                                                    _ptr(self.totals), _ptr(self.morph_ws), self.morph_ws.numel(),
                                                    _ptr(self.morphology), stream), "mb_mask_morphology")
+        # after the masks: a mask overflow flag in totals means nothing is encoded
+        if self.png is not None:
+            self._encode(self.png, self.pixels, stream)
+        if self.mask_png is not None:
+            self._encode(self.mask_png, self.masks, stream)
 
     def checked_totals(self, totals: Optional[Tensor] = None, pixels: bool = True, masks: bool = False) -> List[int]:
         """totals (default: this stage's, one sync; or a host copy of them) as a list, raising if the pixel buffer
@@ -344,6 +383,33 @@ class CropStage:
             raise MisoB200Error(f"mask buffer too small: {tot[1] // self.params.channels} bytes needed, "
                                 f"{self.mask_capacity} available")
         return tot
+
+    @staticmethod
+    def checked_png(buf: dict, what: str = "PNG") -> List[int]:
+        """A PNG buffer's status (one sync) as [total bytes, flag], raising if the buffer or workspace was too small."""
+        st = buf["status"].tolist()
+        if st[1] == 1:
+            raise MisoB200Error(f"{what} buffer too small: {st[0]} bytes needed, {buf['capacity']} available")
+        if st[1]:
+            raise MisoB200Error(f"{what} workspace too small for the crops")
+        return st
+
+    def _png_host(self, buf: Optional[dict], what: str) -> List[bytes]:
+        if buf is None:
+            raise MisoB200Error(f"no {what} streams: bind_png() was not called" + (" after bind_masks()" if "mask" in what else ""))
+        k = self.checked_totals(pixels=buf is self.png, masks=self.masks is not None)[0]
+        total = self.checked_png(buf, what)[0]
+        offs = buf["offsets"][:k + 1].cpu().numpy()
+        data = buf["out"][:total].cpu().numpy().tobytes()
+        return [data[offs[j]:offs[j + 1]] for j in range(k)]
+
+    def png_to_host(self) -> List[bytes]:
+        """Every crop's PNG file as bytes, crop order (b"" for a crop of zero area); one copy of the packed streams."""
+        return self._png_host(self.png, "PNG")
+
+    def mask_png_to_host(self) -> List[bytes]:
+        """Every crop's mask as a PNG file (mode L, 0 / 255), crop order; one copy of the packed streams."""
+        return self._png_host(self.mask_png, "mask PNG")
 
     def to_host(self, channels: int):
         """One device->host transfer; returns per-crop (image index, detection index, xywh, array)."""
@@ -381,7 +447,7 @@ class CropStage:
 def filter_and_crop(images: Sequence[Tensor], det_boxes: Tensor, det_scores: Tensor, det_counts: Tensor,
                     threshold: float, capacity_bytes: Optional[int] = None, boxes_are_xywh: bool = False,
                     mask_probs: Optional[Tensor] = None, paste_boxes: Optional[Tensor] = None, mask_threshold: float = 0.5,
-                    mask_capacity_bytes: Optional[int] = None, morphology: bool = False) -> CropStage:
+                    mask_capacity_bytes: Optional[int] = None, morphology: bool = False, png: bool = False) -> CropStage:
     """images[n]: uint8 [H, W, C] or [H, W] on the device (the ORIGINAL image pixels, as
     skimage.io.imread returns them); det_* as produced by postprocess_detections.
 
@@ -392,7 +458,10 @@ def filter_and_crop(images: Sequence[Tensor], det_boxes: Tensor, det_scores: Ten
 
     morphology=True (needs mask_probs) also measures every crop's mask on the device (mb_mask_morphology): area,
     perimeter, centroid, axes, orientation, eccentricity, equivalent diameter and the mean of each channel over the
-    mask, as regionprops computes them (MORPHOLOGY_FIELDS); CropStage.morphology / morphology_to_host()."""
+    mask, as regionprops computes them (MORPHOLOGY_FIELDS); CropStage.morphology / morphology_to_host().
+
+    png=True also encodes every crop (and mask) as a lossless PNG file on the device (mb_png_encode):
+    CropStage.png_to_host() / mask_png_to_host(). Images of 1..4 channels."""
     if morphology and mask_probs is None:
         raise MisoB200Error("filter_and_crop(morphology=True) measures the instance masks: mask_probs is needed")
     n, cap = det_boxes.shape[0], det_boxes.shape[1]
@@ -422,5 +491,7 @@ def filter_and_crop(images: Sequence[Tensor], det_boxes: Tensor, det_scores: Ten
         torch._assert(pb.numel() == n * cap * 4, "paste_boxes must be [N, cap, 4]")
         stage.bind_masks(mp, pb, None, cap, mask_threshold, need // ch if mask_capacity_bytes is None else mask_capacity_bytes,
                          morphology)
+    if png:
+        stage.bind_png()
     stage.cut(st)
     return stage

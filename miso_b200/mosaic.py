@@ -232,6 +232,10 @@ class MosaicCrops(CropStage):
             out["masks"] = self.masks[:tot[1] // self.params.channels]
             if self.morphology is not None:
                 out["morphology"] = self.morphology[:k]
+        for key, buf in (("png", self.png), ("mask_png", self.mask_png)):
+            if buf is not None:
+                total = self.checked_png(buf, key)[0]
+                out[key], out[key + "_offsets"] = buf["out"][:total], buf["offsets"][:k + 1]
         return out
 
 
@@ -495,7 +499,7 @@ def by_score(gathered: Tensor, state: Tensor) -> Tensor:
 def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: int = 0, tile: int = 1024,
                  overlap: int = 128, threshold: float = 0.5, batch_size: int = 4, rank: int = 0, world: int = 1,
                  group=None, crop_capacity_bytes: int = 256 << 20, masks: bool = False, mask_threshold: float = 0.5,
-                 morphology: bool = False):
+                 morphology: bool = False, png: bool = False):
     """Detect on a large slide/mosaic image (config 5) with a (patched) torchvision detection model: this rank runs
     its contiguous share of tiles, the per-rank detection blocks are exchanged with one all-gather, the sparse seam
     NMS runs on every rank (replicated, deterministic) and each rank cuts the crops of its own tiles' survivors.
@@ -507,7 +511,10 @@ def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: in
     tile it came from, cut to the crop rectangle, > mask_threshold -> 255 (MosaicCrops.bind_masks).
     morphology=True (Mask R-CNN): crops["morphology"] [count, len(MORPHOLOGY_FIELDS)] fp64 on the device, each crop's
     mask measured (area, perimeter, centroid in mosaic coordinates, axes, ...; the masks are cut for it even when
-    masks=False, and crops["masks"] is returned only when masks=True)."""
+    masks=False, and crops["masks"] is returned only when masks=True).
+    png=True: crops["png"] / crops["png_offsets"] hold every crop as a PNG file on the device (packed in crop order,
+    crop j is png[png_offsets[j]:png_offsets[j + 1]]), and crops["mask_png"] / crops["mask_png_offsets"] every mask
+    when masks=True (CropStage.bind_png)."""
     has_mask = getattr(model.roi_heads, "mask_predictor", None) is not None
     if (masks or morphology) and not has_mask:
         what = "masks" if masks else "morphology"
@@ -567,13 +574,20 @@ def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: in
         paste_boxes = torch.zeros((tmax * dpi, 4), dtype=torch.float32, device=dev)
         paste_boxes[:len(mine) * dpi] = boxes[:len(mine)].reshape(-1, 4)
         crops.bind_masks(probs, paste_boxes, frames.to(dev), dpi, mask_threshold, morphology=morphology)
+    if png:
+        crops.bind_png()
     crops.launch(gathered, state, rank * tmax * dpi)
     seam.check()
     res = crops.results()
     if want_masks and probs is None:               # no own tiles: no crops
         res["masks"] = torch.empty((0,), dtype=torch.uint8, device=dev)
+        if png:
+            res["mask_png"] = torch.empty((0,), dtype=torch.uint8, device=dev)
+            res["mask_png_offsets"] = torch.zeros((1,), dtype=torch.int64, device=dev)
         if morphology:
             res["morphology"] = torch.empty((0, len(MORPHOLOGY_FIELDS)), dtype=torch.float64, device=dev)
     if not masks:
         res.pop("masks", None)
+        res.pop("mask_png", None)
+        res.pop("mask_png_offsets", None)
     return {"gathered": gathered, "state": state, "crops": res}
