@@ -759,8 +759,11 @@ static __global__ void __launch_bounds__(kFixThreads) k_nms_fixpoint(SegArrays s
     }
 }
 
-// MB_NMS_SWEEP=blocks keeps the 64-box block sweeps for every segment size (development A/B switch)
-inline bool sweep_in_order() {
+// MB_NMS_SWEEP=blocks keeps the 64-box block sweeps for every segment size (development A/B switch).
+// This helper and launch_mask_and_sweep are static like the kernels: each translation unit that includes this header
+// launches its own copies of the sweep kernels, so it must also keep its own function-local statics (the cached switch,
+// the per-device shared-memory opt-in of MB_DYN_SMEM) instead of sharing one weak definition with the other units.
+static inline bool sweep_in_order() {
     static const bool v = [] { const char* e = getenv("MB_NMS_SWEEP"); return e != nullptr && e[0] == 'b'; }();
     return v;
 }
@@ -768,7 +771,7 @@ inline bool sweep_in_order() {
 inline int sweep_smem_bytes(int max_words) { return max_words * (int)sizeof(unsigned long long); }
 
 // Host helper: launch meta + mask + sweep on prepared sorted boxes.
-inline int launch_mask_and_sweep(const float4* sbox, SegArrays s, int G, int max_seg_elems, double iou_threshold,
+static inline int launch_mask_and_sweep(const float4* sbox, SegArrays s, int G, int max_seg_elems, double iou_threshold,
                                  unsigned long long* mask, unsigned long long* keepbits, int max_keep,
                                  cudaStream_t stream, const float* seg_offset = nullptr) {
     const float thr_up = strict_gt_threshold(iou_threshold);

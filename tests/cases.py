@@ -64,6 +64,66 @@ def batched_nms_cases():
     return out
 
 
+NMS_FAMILIES = ("random", "chain", "cluster", "ties", "zero_area")
+
+
+def nms_family(family, n, thr, seed=0):
+    """(boxes [n, 4], scores [n]) of one NMS input family, seeded by (family, n, seed):
+    random     boxes spread so that most are disjoint, distinct scores;
+    chain      suppression chains: link k overlaps k - 1 above thr and k - 2 at most at thr, scores falling along the
+               chain, so keep / remove alternate. The first chain runs through min(n, 1024) consecutive score ranks (the
+               fixed-point sweep's worst case, n rounds); the others are interleaved in score order, so that every link
+               crosses 64-box blocks of the sorted order;
+    cluster    a dense cluster in which every box overlaps dozens of others;
+    ties       scores quantised to 1/64 around 0, with NaN, +0 and -0 among them;
+    zero_area  random boxes with exact duplicates, zero-area boxes and zero-area duplicates (0/0 IoU)."""
+    rng = np.random.default_rng([NMS_FAMILIES.index(family), n, seed])
+    if family == "random":
+        return random_boxes(rng, n, extent=16.0 * np.sqrt(n) + 64.0), distinct_scores(rng, n)
+    if family == "cluster":
+        return random_boxes(rng, n, extent=10.0 * np.sqrt(n) + 48.0, wh=(24.0, 48.0)), distinct_scores(rng, n)
+    if family == "ties":
+        b = random_boxes(rng, n, extent=8.0 * np.sqrt(n) + 64.0)
+        s = (np.floor(rng.uniform(-1, 1, n) * 64) / 64).astype(F)
+        s[rng.integers(0, n, max(1, n // 50))] = np.nan
+        s[rng.integers(0, n, max(1, n // 50))] = 0.0
+        s[rng.integers(0, n, max(1, n // 50))] = -0.0
+        return b, s
+    if family == "zero_area":
+        b = random_boxes(rng, n, extent=12.0 * np.sqrt(n) + 64.0)
+        q = rng.permutation(n)
+        k = n // 6
+        b[q[:k]] = b[q[k:2 * k]]                                            # exact duplicates: IoU 1
+        b[q[2 * k:3 * k], 2] = b[q[2 * k:3 * k], 0]                         # zero width
+        z = q[3 * k:3 * k + k // 2]
+        b[z] = np.repeat(np.array([[7.0, 7.0, 7.0, 7.0]], F), len(z), axis=0)   # zero-area duplicates: NaN IoU
+        return b.astype(F), distinct_scores(rng, n)
+    assert family == "chain", family
+    # link step d: IoU(d) = (w - d) / (w + d) > t >= IoU(2 d) for d = 3/4 of the step at which IoU == t
+    w = 16.0
+    t = min(max(float(thr), 0.0), 0.9)
+    d = 0.75 * w * (1.0 - t) / (1.0 + t)
+    first = min(n, 1024)
+    rest = n - first
+    nchains = max(1, min(64, rest // 16)) if rest else 0
+    b = np.zeros((n, 4), F)
+    rank = np.zeros(n, np.int64)
+    b[:first, 0] = np.arange(first) * d
+    b[:first, 1] = 0.0
+    rank[:first] = np.arange(first)
+    if rest:
+        c = np.arange(rest) % nchains                                       # chain of box first + i
+        k = np.arange(rest) // nchains                                      # position along it
+        b[first:, 0] = k * d
+        b[first:, 1] = 2.0 * w * (c + 1)
+        rank[first:] = first + np.arange(rest)                              # chains interleaved in score order
+    b[:, 2] = b[:, 0] + w
+    b[:, 3] = b[:, 1] + w
+    perm = rng.permutation(n)                                               # storage order unrelated to score order
+    scores = (1.0 - (rank.astype(np.float64) + 1.0) / (n + 1.0)).astype(F)
+    return b[perm], scores[perm]
+
+
 ROI_GOLDEN_CHANNELS = [0, 13, 39]
 
 
