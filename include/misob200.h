@@ -367,6 +367,45 @@ int mb_png_encode(const mb_crop_params* params_host, const uint8_t* packed, int3
                   const int64_t* offsets, const int64_t* totals, void* workspace, size_t workspace_bytes,
                   uint8_t* png_out, int64_t png_capacity_bytes, int64_t* png_offsets_out, int64_t* png_status_out,
                   mb_stream_t stream);
+/* Baseline JPEG files of the packed crops (mb_crop_gather), channels 1 (mode L) or 3 (RGB): one complete file per crop,
+ * packed in crop order at jpeg_offsets_out[j] ([num_images*capacity + 1] int64; 0 bytes when h*w == 0). Crop j (rect
+ * (x, y, w, h)) is read at packed + offsets[j] / params.channels * channels. The file is byte for byte what
+ * PIL.Image.fromarray(crop).save(f, "JPEG") writes with default arguments (libjpeg-turbo):
+ *   framing  SOI; APP0 JFIF 1.1, no units, density 1:1, no thumbnail; DQT luminance (and chrominance for 3 channels);
+ *            SOF0 (8 bit, h, w; components 1, 2, 3 with sampling 0x22, 0x11, 0x11 and tables 0, 1, 1, or one
+ *            component 0x11); DHT DC0, AC0 (and DC1, AC1), the Annex K tables; SOS over 0..63; the scan; EOI. No
+ *            other markers, no restart intervals. Headers are 328 (grey) and 623 (colour) bytes.
+ *   quant    Annex K tables at quality 75: q = clamp((std * 50 + 50) / 100, 1, 255), written in zigzag order
+ *   colour   jccolor.c with FIX(x) = (int)(x * 65536 + 0.5): Y = (FIX(.299) r + FIX(.587) g + FIX(.114) b + 2^15) >> 16,
+ *            Cb = (-FIX(.16874) r - FIX(.33126) g + FIX(.5) b + (128 << 16) + 2^15 - 1) >> 16,
+ *            Cr = (FIX(.5) r - FIX(.41869) g - FIX(.08131) b + (128 << 16) + 2^15 - 1) >> 16
+ *   edges    luma padded to 8 ceil(w/8) x 8 ceil(h/8) by replicating the last column and row; chroma: the full-resolution
+ *            plane padded by replication to 2 ceil(h/2) rows and 16 ceil(ceil(w/2)/8) columns, downsampled 2x2 as
+ *            (sum of 4 + bias) >> 2 with bias 1, 2, 1, 2, ... along each output row, then the downsampled rows padded
+ *            by replication to a whole block row
+ *   DCT      jfdctint.c islow on samples - 128: rows (PASS1_BITS 2), then columns; CONST_BITS 13,
+ *            DESCALE(x, n) = (x + 2^(n-1)) >> n; quantised as (|c| + 4q) / 8q with the sign of c
+ *   scan     MCU 16x16 (Y0 Y1 Y2 Y3 Cb Cr) or one 8x8 block; a DC predictor per component from 0; blocks of an MCU past
+ *            the component's last real block column or row are dummy blocks (zero AC, the DC of the block before
+ *            them in the MCU); Huffman codes with ZRL and EOB, negative amplitudes v + 2^n - 1, 0x00 after every 0xFF
+ *            data byte, the last byte padded with 1-bits
+ * mb_jpeg_bound_bytes: a capacity no packed set of `crops` crops of packed_bytes bytes can exceed: every block at
+ *   1660 bits (DC <= 11 + 11, each AC <= 16 + 10) and every data byte stuffed, on crops 1 pixel wide, which have the
+ *   most blocks per pixel: crops * (H + 2) + 416 * B with H the header bytes and, for P = packed_bytes / channels
+ *   pixels, B = P / 8 + crops (grey) or 6 * (P / 16 + crops) (colour); -1 for bad input.
+ * mb_jpeg_workspace_bytes: enough for any packed crops of up to packed_capacity_bytes: 16 B of record per block plus
+ *   its unstuffed codes (at most 208 B), B blocks as above, plus 40 B per slot. The codes take their exact size, so
+ *   less suffices for real content (large photographic crops need about 0.5 B per pixel: 16 B per 64 or 43 pixels
+ *   plus the file size); a workspace too small for the crops at hand sets flag 2.
+ * jpeg_status_out [2] int64: [0] total bytes, [1] 1 if that exceeds jpeg_capacity_bytes (nothing is written), 2 if the
+ * workspace is too small for the crops (nothing is encoded), else 0. A pixel overflow flag in totals (totals[2]) means
+ * nothing is encoded (no crops). Channels other than 1 or 3, or an image side above 65535: MB_ERR_UNSUPPORTED. */
+int64_t mb_jpeg_bound_bytes(int64_t packed_bytes, int64_t crops, int32_t channels);
+size_t mb_jpeg_workspace_bytes(const mb_crop_params* params_host, int64_t packed_capacity_bytes, int32_t channels);
+int mb_jpeg_encode(const mb_crop_params* params_host, const uint8_t* packed, int32_t channels, const int32_t* rects,
+                   const int64_t* offsets, const int64_t* totals, void* workspace, size_t workspace_bytes,
+                   uint8_t* jpeg_out, int64_t jpeg_capacity_bytes, int64_t* jpeg_offsets_out, int64_t* jpeg_status_out,
+                   mb_stream_t stream);
 /* maskrcnn_inference (tv:models/detection/roi_heads.py:56-82): mask_logits [R, C, M, M], labels [R] int64 ->
  * out [R, 1, M, M] = sigmoid(mask_logits[r, labels[r]]). Labels outside [0, C) are the caller's error. */
 int mb_mask_prob(const float* mask_logits, const int64_t* labels, int64_t num_masks, int32_t num_classes,

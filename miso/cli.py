@@ -86,8 +86,11 @@ def crop_objects(tasks, output_dir, wsl2, api):
 @click.option('--png-on-gpu', is_flag=True, default=False,
               help='Encode the crops of 8-bit PNG images on the GPU (lossless: the same pixels as the default files, '
                    'other bytes); other formats and the mask files are encoded on the CPU')
+@click.option('--jpeg-on-gpu', is_flag=True, default=False,
+              help='Encode the crops of 8-bit grey / RGB JPEG images on the GPU (byte for byte the default files); '
+                   'other formats are encoded on the CPU')
 def infer_object_detector_directory(input_dir, output_dir, model_dir, model, threshold, batch_size, mask_dir, morphology_csv,
-                                    png_on_gpu):
+                                    png_on_gpu, jpeg_on_gpu):
     model_path = os.path.join(model_dir, model, "model.pt")
     labels = read_labels(os.path.join(model_dir, model, "labels.txt"))
     if mask_dir is None and morphology_csv is None:
@@ -100,7 +103,7 @@ def infer_object_detector_directory(input_dir, output_dir, model_dir, model, thr
             raise click.ClickException(str(e))
     Path(output_dir).mkdir(parents=True, exist_ok=True)
     crop_objects_fn(project, output_dir, relative_to=input_dir, mask_dir=mask_dir, morphology_csv=morphology_csv,
-                    png_on_gpu=png_on_gpu)
+                    png_on_gpu=png_on_gpu, jpeg_on_gpu=jpeg_on_gpu)
 
 
 if __name__ == "__main__":

@@ -25,7 +25,7 @@ def _imread(path: str) -> np.ndarray:
 
 
 def crop_objects(project: Project, output_dir: str, relative_to=None, mask_dir=None, morphology_csv=None,
-                 png_on_gpu=False):
+                 png_on_gpu=False, jpeg_on_gpu=False):
     """Crops of every annotation under output_dir/<sub-folders>/<label>/. With mask_dir, each annotation's instance mask
     (`mask`, set by inference with_masks=True) is written as well, as a PNG (mode L, 0 / 255) with the crop's relative
     path and file name under mask_dir — a separate tree, so classifiers trained on the crop folders never see it.
@@ -35,7 +35,10 @@ def crop_objects(project: Project, output_dir: str, relative_to=None, mask_dir=N
     Numbers are written with repr, so they read back exactly; values are in pixels.
     png_on_gpu=True encodes the crops of .png sources (any case) that are uint8 with 1..4 channels on the device
     (mb_png_encode, lossless: the same pixels as PIL's files, other bytes); the pool then only writes the files. Other
-    sources and the mask files keep PIL."""
+    sources and the mask files keep PIL.
+    jpeg_on_gpu=True encodes the crops of .jpg / .jpeg sources (any case) that are uint8 with 1 or 3 channels on the
+    device (mb_jpeg_encode): byte for byte the files PIL writes by default. Other sources (CMYK JPEGs, PNG, TIFF, 16-bit)
+    keep their path; the two options are independent."""
     from PIL import Image
     from miso_b200 import detection
     os.makedirs(output_dir, exist_ok=True)
@@ -72,10 +75,13 @@ def crop_objects(project: Project, output_dir: str, relative_to=None, mask_dir=N
         scores = torch.ones((1, k), dtype=torch.float32, device="cuda")
         counts = torch.tensor([k], dtype=torch.int32, device="cuda")
         path = Path(image.full_path)
-        on_gpu = png_on_gpu and path.suffix.lower() == ".png" and im.dtype == np.uint8 and 1 <= bpp <= 4
+        suffix = path.suffix.lower()
+        on_gpu = png_on_gpu and suffix == ".png" and im.dtype == np.uint8 and 1 <= bpp <= 4
+        jpeg_gpu = jpeg_on_gpu and suffix in (".jpg", ".jpeg") and im.dtype == np.uint8 and bpp in (1, 3)
         out = detection.filter_and_crop([dev], bounds[None], scores, counts, 0.5, boxes_are_xywh=False,
-                                        **({"png": True} if on_gpu else {}))
-        encoded = out.png_to_host() if on_gpu else None
+                                        **({"png": True} if on_gpu else {}), **({"jpeg": True} if jpeg_gpu else {}))
+        encoded = out.png_to_host() if on_gpu else out.jpeg_to_host() if jpeg_gpu else None
+        on_gpu = on_gpu or jpeg_gpu
         crops = [(n, i, xywh, np.ascontiguousarray(c).reshape(c.shape[0], c.shape[1], bpp).view(im.dtype).reshape(c.shape[:2] + px_shape))
                  for n, i, xywh, c in out.to_host(bpp)]
         for j, ((_, idx, _xywh, crop), box) in enumerate(zip(crops, image.boxes)):

@@ -119,6 +119,9 @@ SIGNATURES = {
     "mb_png_bound_bytes": (_i64, [_i64, _i64, _i32]),
     "mb_png_workspace_bytes": (_sz, [C.POINTER(CropParams), _i64, _i32]),
     "mb_png_encode": (C.c_int, [C.POINTER(CropParams), _p, _i32, _p, _p, _p, _p, _sz, _p, _i64, _p, _p, _p]),
+    "mb_jpeg_bound_bytes": (_i64, [_i64, _i64, _i32]),
+    "mb_jpeg_workspace_bytes": (_sz, [C.POINTER(CropParams), _i64, _i32]),
+    "mb_jpeg_encode": (C.c_int, [C.POINTER(CropParams), _p, _i32, _p, _p, _p, _p, _sz, _p, _i64, _p, _p, _p]),
     "mb_image_transform": (C.c_int, [C.POINTER(TransformParams), _p, _p]),
 }
 

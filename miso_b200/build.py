@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 LIB = os.path.join(HERE, "libmisob200.so")
 STAMP = os.path.join(HERE, ".libmisob200.stamp")
-SOURCES = ["api.cu", "nms.cu", "roi_align.cu", "roi_align_tma.cu", "boxops.cu", "rpn.cu", "detpost.cu", "crop.cu", "mosaic.cu", "seam.cu", "train.cu", "paste.cu", "morph.cu", "png.cu", "transform.cu"]
+SOURCES = ["api.cu", "nms.cu", "roi_align.cu", "roi_align_tma.cu", "boxops.cu", "rpn.cu", "detpost.cu", "crop.cu", "mosaic.cu", "seam.cu", "train.cu", "paste.cu", "morph.cu", "png.cu", "jpeg.cu", "transform.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

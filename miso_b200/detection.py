@@ -267,6 +267,7 @@ class CropStage:
       morphology  [N*cap, len(MORPHOLOGY_FIELDS)] fp64 records (bind_masks(morphology=True))
       png, png_offsets, png_status          one PNG file per crop, packed in crop order (bind_png(), mb_png_encode);
       mask_png, mask_png_offsets, mask_png_status   the same for the masks (bind_png() with bind_masks())
+      jpeg        one JPEG file per crop, packed in crop order, the bytes PIL writes by default (bind_jpeg(), mb_jpeg_encode)
     """
 
     def __init__(self, image_hw: Sequence[Tuple[int, int]], channels: int, capacity: int, threshold: float, device,
@@ -285,7 +286,7 @@ class CropStage:
         self.mask_args = self.masks = self.morphology = self.morph_ws = None
         self.capacity = self.mask_capacity = 0
         self.pixels = None
-        self.png = self.mask_png = None
+        self.png = self.mask_png = self.jpeg = None
         if capacity_bytes is not None:
             self.reserve(capacity_bytes)
 
@@ -325,24 +326,33 @@ class CropStage:
         if self.masks is not None:
             self.mask_png = self._png_buffers(self.mask_capacity, 1, mask_capacity_bytes)
 
-    def _png_buffers(self, packed_capacity: int, channels: int, capacity_bytes: Optional[int]) -> dict:
+    def bind_jpeg(self, capacity_bytes: Optional[int] = None) -> None:
+        """Encode every crop as a JPEG file after the gather (mb_jpeg_encode): the bytes PIL's Image.save writes with
+        default settings. 1 or 3 channels. The capacity defaults to mb_jpeg_bound_bytes of the pixel buffer, which no
+        crop set can exceed (416 B per 8x8 block of 1-pixel-wide crops); pass a smaller one to save memory, an overflow
+        is then reported by jpeg_to_host()."""
+        self.jpeg = self._png_buffers(self.capacity, self.params.channels, capacity_bytes, "jpeg")
+
+    def _png_buffers(self, packed_capacity: int, channels: int, capacity_bytes: Optional[int], kind: str = "png") -> dict:
         slots = self.rects.shape[0]
         if capacity_bytes is None:
-            capacity_bytes = int(self.lib.mb_png_bound_bytes(packed_capacity, slots, channels))
-        ws = int(self.lib.mb_png_workspace_bytes(C.byref(self.params), packed_capacity, channels))
+            capacity_bytes = int(getattr(self.lib, f"mb_{kind}_bound_bytes")(packed_capacity, slots, channels))
+        ws = int(getattr(self.lib, f"mb_{kind}_workspace_bytes")(C.byref(self.params), packed_capacity, channels))
         if capacity_bytes < 0 or ws == 0:
-            raise MisoB200Error(f"mb_png_encode: {channels} channels are not supported (1..4)")
-        return {"channels": channels, "capacity": int(capacity_bytes),
+            raise MisoB200Error(f"mb_{kind}_encode: {channels} channels are not supported "
+                                f"({'1..4' if kind == 'png' else '1 or 3'})")
+        return {"kind": kind, "channels": channels, "capacity": int(capacity_bytes),
                 "out": torch.empty((max(int(capacity_bytes), 1),), dtype=torch.uint8, device=self.dev),
                 "offsets": torch.zeros((slots + 1,), dtype=torch.int64, device=self.dev),
                 "status": torch.zeros((2,), dtype=torch.int64, device=self.dev),
                 "ws": torch.empty((ws,), dtype=torch.uint8, device=self.dev)}
 
     def _encode(self, buf: dict, packed: Tensor, stream) -> None:
-        _lib.check(self.lib.mb_png_encode(C.byref(self.params), _ptr(packed), buf["channels"], _ptr(self.rects),
-                                          _ptr(self.offsets), _ptr(self.totals), _ptr(buf["ws"]), buf["ws"].numel(),
-                                          _ptr(buf["out"]), buf["capacity"], _ptr(buf["offsets"]), _ptr(buf["status"]),
-                                          stream), "mb_png_encode")
+        fn = f"mb_{buf['kind']}_encode"
+        _lib.check(getattr(self.lib, fn)(C.byref(self.params), _ptr(packed), buf["channels"], _ptr(self.rects),
+                                         _ptr(self.offsets), _ptr(self.totals), _ptr(buf["ws"]), buf["ws"].numel(),
+                                         _ptr(buf["out"]), buf["capacity"], _ptr(buf["offsets"]), _ptr(buf["status"]),
+                                         stream), fn)
 
     def plan(self, boxes: Tensor, scores: Tensor, counts: Tensor, stream) -> None:
         """mb_crop_plan: boxes [N, cap, 4] fp32, scores [N, cap] fp32, counts [N] int32, all contiguous."""
@@ -355,6 +365,8 @@ class CropStage:
         cp = C.byref(self.params)
         _lib.check(self.lib.mb_crop_gather(cp, _ptr(self.rects), _ptr(self.src), _ptr(self.offsets), _ptr(self.totals),
                                            _ptr(self.pixels), self.capacity, stream), "mb_crop_gather")
+        if self.jpeg is not None:
+            self._encode(self.jpeg, self.pixels, stream)
         if self.mask_args is None:
             if self.png is not None:
                 self._encode(self.png, self.pixels, stream)
@@ -396,8 +408,10 @@ class CropStage:
 
     def _png_host(self, buf: Optional[dict], what: str) -> List[bytes]:
         if buf is None:
-            raise MisoB200Error(f"no {what} streams: bind_png() was not called" + (" after bind_masks()" if "mask" in what else ""))
-        k = self.checked_totals(pixels=buf is self.png, masks=self.masks is not None)[0]
+            bind = "bind_jpeg()" if what == "JPEG" else "bind_png()"
+            raise MisoB200Error(f"no {what} streams: {bind} was not called" + (" after bind_masks()" if "mask" in what else ""))
+        # the PNG encoder skips every crop on a mask overflow, the JPEG encoder only on a pixel overflow
+        k = self.checked_totals(pixels=buf is not self.mask_png, masks=buf is not self.jpeg and self.masks is not None)[0]
         total = self.checked_png(buf, what)[0]
         offs = buf["offsets"][:k + 1].cpu().numpy()
         data = buf["out"][:total].cpu().numpy().tobytes()
@@ -406,6 +420,10 @@ class CropStage:
     def png_to_host(self) -> List[bytes]:
         """Every crop's PNG file as bytes, crop order (b"" for a crop of zero area); one copy of the packed streams."""
         return self._png_host(self.png, "PNG")
+
+    def jpeg_to_host(self) -> List[bytes]:
+        """Every crop's JPEG file as bytes, crop order (b"" for a crop of zero area); one copy of the packed streams."""
+        return self._png_host(self.jpeg, "JPEG")
 
     def mask_png_to_host(self) -> List[bytes]:
         """Every crop's mask as a PNG file (mode L, 0 / 255), crop order; one copy of the packed streams."""
@@ -447,7 +465,8 @@ class CropStage:
 def filter_and_crop(images: Sequence[Tensor], det_boxes: Tensor, det_scores: Tensor, det_counts: Tensor,
                     threshold: float, capacity_bytes: Optional[int] = None, boxes_are_xywh: bool = False,
                     mask_probs: Optional[Tensor] = None, paste_boxes: Optional[Tensor] = None, mask_threshold: float = 0.5,
-                    mask_capacity_bytes: Optional[int] = None, morphology: bool = False, png: bool = False) -> CropStage:
+                    mask_capacity_bytes: Optional[int] = None, morphology: bool = False, png: bool = False,
+                    jpeg: bool = False) -> CropStage:
     """images[n]: uint8 [H, W, C] or [H, W] on the device (the ORIGINAL image pixels, as
     skimage.io.imread returns them); det_* as produced by postprocess_detections.
 
@@ -461,7 +480,10 @@ def filter_and_crop(images: Sequence[Tensor], det_boxes: Tensor, det_scores: Ten
     mask, as regionprops computes them (MORPHOLOGY_FIELDS); CropStage.morphology / morphology_to_host().
 
     png=True also encodes every crop (and mask) as a lossless PNG file on the device (mb_png_encode):
-    CropStage.png_to_host() / mask_png_to_host(). Images of 1..4 channels."""
+    CropStage.png_to_host() / mask_png_to_host(). Images of 1..4 channels.
+
+    jpeg=True also encodes every crop as a JPEG file on the device (mb_jpeg_encode), byte for byte the file PIL's
+    Image.save writes with default settings: CropStage.jpeg_to_host(). Images of 1 or 3 channels."""
     if morphology and mask_probs is None:
         raise MisoB200Error("filter_and_crop(morphology=True) measures the instance masks: mask_probs is needed")
     n, cap = det_boxes.shape[0], det_boxes.shape[1]
@@ -493,5 +515,7 @@ def filter_and_crop(images: Sequence[Tensor], det_boxes: Tensor, det_scores: Ten
                          morphology)
     if png:
         stage.bind_png()
+    if jpeg:
+        stage.bind_jpeg()
     stage.cut(st)
     return stage

@@ -232,7 +232,7 @@ class MosaicCrops(CropStage):
             out["masks"] = self.masks[:tot[1] // self.params.channels]
             if self.morphology is not None:
                 out["morphology"] = self.morphology[:k]
-        for key, buf in (("png", self.png), ("mask_png", self.mask_png)):
+        for key, buf in (("png", self.png), ("mask_png", self.mask_png), ("jpeg", self.jpeg)):
             if buf is not None:
                 total = self.checked_png(buf, key)[0]
                 out[key], out[key + "_offsets"] = buf["out"][:total], buf["offsets"][:k + 1]
@@ -499,7 +499,7 @@ def by_score(gathered: Tensor, state: Tensor) -> Tensor:
 def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: int = 0, tile: int = 1024,
                  overlap: int = 128, threshold: float = 0.5, batch_size: int = 4, rank: int = 0, world: int = 1,
                  group=None, crop_capacity_bytes: int = 256 << 20, masks: bool = False, mask_threshold: float = 0.5,
-                 morphology: bool = False, png: bool = False):
+                 morphology: bool = False, png: bool = False, jpeg: bool = False):
     """Detect on a large slide/mosaic image (config 5) with a (patched) torchvision detection model: this rank runs
     its contiguous share of tiles, the per-rank detection blocks are exchanged with one all-gather, the sparse seam
     NMS runs on every rank (replicated, deterministic) and each rank cuts the crops of its own tiles' survivors.
@@ -514,7 +514,9 @@ def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: in
     masks=False, and crops["masks"] is returned only when masks=True).
     png=True: crops["png"] / crops["png_offsets"] hold every crop as a PNG file on the device (packed in crop order,
     crop j is png[png_offsets[j]:png_offsets[j + 1]]), and crops["mask_png"] / crops["mask_png_offsets"] every mask
-    when masks=True (CropStage.bind_png)."""
+    when masks=True (CropStage.bind_png).
+    jpeg=True: crops["jpeg"] / crops["jpeg_offsets"] hold every crop as a JPEG file on the device, byte for byte what PIL
+    writes with default settings (packed in crop order, CropStage.bind_jpeg); 1 or 3 channels."""
     has_mask = getattr(model.roi_heads, "mask_predictor", None) is not None
     if (masks or morphology) and not has_mask:
         what = "masks" if masks else "morphology"
@@ -576,6 +578,8 @@ def infer_mosaic(model, band_u8: Tensor, mosaic_hw: Tuple[int, int], band_y0: in
         crops.bind_masks(probs, paste_boxes, frames.to(dev), dpi, mask_threshold, morphology=morphology)
     if png:
         crops.bind_png()
+    if jpeg:
+        crops.bind_jpeg()
     crops.launch(gathered, state, rank * tmax * dpi)
     seam.check()
     res = crops.results()
